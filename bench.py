@@ -2,6 +2,7 @@
 """Headline benchmark: SNN-detector training throughput (images/s) on B200 through the libsnnb200 hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]                 # our arm (1 GPU, or under torchrun: N ranks)
+    python bench.py --dump-outputs DIR                                  # + the last timed step's results as DIR/*.npy
     python bench.py --impl reference [--steps K] [--warmup W]           # CPU arm: oracle port of the reference path
     python bench.py --impl eager-gpu                                    # GPU comparator: the oracle modules in PyTorch eager
     python bench.py --microbench lif                                    # BASELINE.json configs[3] LIF sweep (GB/s)
@@ -18,7 +19,8 @@ right after the timed region, matched launch by launch to the ABI calls recorded
 around eager launches), `cfg3` = the same measurement on BASELINE.json configs[2] (T=8, 512x512, batch 16/GPU) so that
 the scaling runs carry it at every N, `ranks_in_lockstep` = every rank holds bit-identical parameters after the timed
 steps, `cpu_baseline` = the oracle port of the reference path on this box's host cores and `gpu_eager_baseline` = the
-same oracle modules in PyTorch eager on this GPU (N=1 only), `lif_microbench` = configs[3] sweep with its own clocks.
+same oracle modules in PyTorch eager on this GPU (N=1 only), `lif_microbench` = configs[3] sweep with its own clocks
+(worst fractions only; `--microbench lif` prints the rows).
 """
 import argparse
 import json
@@ -41,7 +43,8 @@ MAX_LR, WEIGHT_DECAY = 1e-4, 5e-4                               # config.yaml:23
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed training steps of the measured path (the baseline sub-records "
+                    "of a single-GPU run use fixed counts: 3 timed + 2 warm-up steps on the GPU, 3 + 1 on the CPU)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "eager-gpu"])
     ap.add_argument("--config", type=int, default=2, choices=[1, 2, 3], help="BASELINE.json configs index + 1")
@@ -57,6 +60,9 @@ def parse():
     ap.add_argument("--no-lif", action="store_true", help="skip the configs[3] LIF sweep sub-record")
     ap.add_argument("--no-gpu-eager", action="store_true", help="skip the PyTorch-eager GPU comparator")
     ap.add_argument("--dump-trace", default=None, help="write the ABI call sequence of one training step (name, work, shape tag) as JSON")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the last one's loss, loss items, gradient norm and a seeded sample of "
+                         "the updated parameters as DIR/<name>.npy (float32)")
     return ap.parse_args()
 
 
@@ -293,7 +299,7 @@ def run_gpu_eager(args):
         return
     torch.cuda.set_device(0)
     B, T, HW = workload(args)
-    r = gpu_eager_run(T, HW, B, max(2, min(args.steps, 5)), 2, args.neuron, torch.device("cuda", 0))
+    r = gpu_eager_run(T, HW, B, args.steps, args.warmup, args.neuron, torch.device("cuda", 0))
     best = max((v for v in (r.get("fp32"), r.get("bf16_autocast")) if v and "value" in v), key=lambda v: v["value"])
     print(json.dumps({"impl": "eager-gpu", "metric": "train images/sec", "value": best["value"], "unit": "images/s", "n_gpus": 1,
                       "steps": args.steps, "warmup": args.warmup, "ms_per_step": best["ms_per_step"], "higher_is_better": True,
@@ -454,6 +460,27 @@ def summarize(agg, shapes, steps, pk):
     return out, by_shape
 
 
+DUMP_PARAM_SAMPLES = 1 << 22          # 16 MB of float32 out of the model's ~120 M parameters
+
+
+def dump_outputs(out_dir, loss, items, grad_norm, model):
+    """What one training step hands back, as float32 .npy files: the loss vector it returns (loss * B and the detached
+    box / cls / dfl items), the gradient norm it clipped with, and the parameters its optimizer step wrote.  Parameters
+    are taken over model.parameters() in declaration order; above DUMP_PARAM_SAMPLES of them, at positions drawn from a
+    fixed seed, so that two builds of the same model are compared at the same weights."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    params = torch.cat([p.detach().reshape(-1).float() for p in model.parameters()])
+    if params.numel() > DUMP_PARAM_SAMPLES:
+        g = torch.Generator().manual_seed(0)
+        idx = torch.randint(0, params.numel(), (DUMP_PARAM_SAMPLES,), generator=g).sort().values
+        params = params[idx.to(params.device)]
+    arrays = {"loss": loss, "loss_items": items, "grad_norm": grad_norm, "params_sample": params}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------
 # our arm: one configuration
 # ------------------------------------------------------------------------------------------------
@@ -523,6 +550,9 @@ def measure_config(args, cfg_idx, dev, rank, local, world, pk, full):
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_total = float(ms)
     last_loss = [float(v) for v in items]
+    # before the accounting replays below: a graphed step returns the graph's static buffers, which every replay overwrites
+    if args.dump_outputs and full and rank == 0:
+        dump_outputs(args.dump_outputs, loss, items, trainer.grad_norm, model)
 
     # ---------------- per-kernel accounting + roofline of the dominant kernel ----------------
     # (done right after the timed region, before the e2e leg re-captures the graph for uint8 host frames)
@@ -697,8 +727,31 @@ def run_ours(args):
         "kernel_ms_sum_per_step": main["kernel_ms_sum"], "other_kernels_ms_per_step": main["other_kernels"],
         "comm_timeline": main["comm_timeline"], "lif_microbench": lif, "last_loss_items": main["last_loss"],
     }
-    print(json.dumps(line), flush=True)
+    print(result_line(line), flush=True)
     shutdown()
+
+
+RESULT_LINE_MAX = 8192       # bytes: readers of the result line keep a bounded tail of stdout (a 21 KB line arrived cut)
+
+
+def result_line(rec):
+    """The one JSON result line of the record: without the per-row LIF sweep (`--microbench lif` prints the rows), the
+    per-shape kernel table cut to its 8 costliest entries and floats kept to 6 significant digits, which holds a
+    single-GPU record below RESULT_LINE_MAX."""
+    def r6(o):
+        if isinstance(o, float):
+            return float(f"{o:.6g}")
+        if isinstance(o, dict):
+            return {k: r6(v) for k, v in o.items()}
+        if isinstance(o, list):
+            return [r6(v) for v in o]
+        return o
+    rec = dict(rec)
+    if rec.get("kernels_by_shape"):
+        rec["kernels_by_shape"] = rec["kernels_by_shape"][:8]
+    if rec.get("lif_microbench"):
+        rec["lif_microbench"] = {k: v for k, v in rec["lif_microbench"].items() if k != "rows"}
+    return json.dumps(r6(rec))
 
 
 # ------------------------------------------------------------------------------------------------

@@ -9,7 +9,8 @@ stubbed) and records inputs/outputs/gradients of the reference's own classes:
                      (reference model.py:9-71), train- and eval-mode BN, forward + backward.
 * ref_unet_seq_256.pt -- same as ref_unet_seq.pt at the geometry of BASELINE.json configs[0] (B=2, T=4, feature
                      maps 32/16/8 of a 256x256 frame); BatchNorm groups are >= 32 samples there, so bf16-operand
-                     kernels can be compared against it at a meaningful tolerance.
+                     kernels can be compared against it at a meaningful tolerance.  Its output maps are stored as
+                     sampled() records (norm, max |x| and a 1-in-7 strided sample), which keeps the file under 1 MB.
 * ref_unet_seq.pt -- full-width TemporalUNet([144,144,144]) (model.py:100-146) initialised with
                      initialize_weights (weight_initialization.py:8-56) under torch.manual_seed(42),
                      T=3 unroll with ConvLSTM state carry (train.py:62-66), loss on the last step,
@@ -30,6 +31,15 @@ sys.path.insert(0, ROOT)
 from oracle.ref_loader import load_reference  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
+OUT_STRIDE = 7
+
+
+def sampled(t):
+    """{shape, norm, absmax, sample}: the whole tensor's shape, norm and max |x|, and an OUT_STRIDE strided sample of it
+    flattened."""
+    t = t.detach().float()
+    return dict(shape=tuple(t.shape), norm=float(t.double().norm()), absmax=float(t.abs().max()),
+                sample=t.flatten()[::OUT_STRIDE].clone())
 
 
 def blocks(ref):
@@ -105,7 +115,7 @@ def blocks(ref):
     print("ref_blocks.pt", os.path.getsize(os.path.join(OUT, "ref_blocks.pt")))
 
 
-def unet_seq(ref, wi, name="ref_unet_seq.pt", B=2, T=3, hw=(8, 4, 2), feat_seed=4242, store_outs=True):
+def unet_seq(ref, wi, name="ref_unet_seq.pt", B=2, T=3, hw=(8, 4, 2), feat_seed=4242, sample_outs=False):
     torch.manual_seed(42)
     net = ref.TemporalUNet([144, 144, 144], use_conv_lstm=True)
     net.apply(wi.initialize_weights)
@@ -120,8 +130,8 @@ def unet_seq(ref, wi, name="ref_unet_seq.pt", B=2, T=3, hw=(8, 4, 2), feat_seed=
         outs, hid = net(f, hid)
     loss = sum((o ** 2).mean() for o in outs)
     loss.backward()
-    fx = dict(B=B, T=T, hw=hw, feat_seed=feat_seed, init_seed=42, init_checksums=init_ck,
-              outs=[o.detach().clone() for o in outs], h=hid[0].detach().clone(), c=hid[1].detach().clone(),
+    fx = dict(B=B, T=T, hw=hw, feat_seed=feat_seed, init_seed=42, init_checksums=init_ck, out_stride=OUT_STRIDE,
+              outs=[sampled(o) if sample_outs else o.detach().clone() for o in outs], h=hid[0].detach().clone(), c=hid[1].detach().clone(),
               loss=float(loss),
               grad_norms={k: float(p.grad.double().norm()) for k, p in net.named_parameters()},
               bn_running={k: v.clone() for k, v in net.state_dict().items() if "running" in k and v.numel() <= 256},
@@ -130,7 +140,7 @@ def unet_seq(ref, wi, name="ref_unet_seq.pt", B=2, T=3, hw=(8, 4, 2), feat_seed=
     net.eval()
     with torch.no_grad():
         eo, _ = net(feats[0], None)
-    fx["eval_outs"] = [o.clone() for o in eo]
+    fx["eval_outs"] = [sampled(o) if sample_outs else o.clone() for o in eo]
     torch.save(fx, os.path.join(OUT, name))
     print(name, os.path.getsize(os.path.join(OUT, name)))
 
@@ -141,4 +151,4 @@ if __name__ == "__main__":
     blocks(ref)
     unet_seq(ref, wi)
     # BASELINE.json configs[0] geometry: B=2, T=4, 256x256 frames -> feature maps 32/16/8, bottleneck 4x4
-    unet_seq(ref, wi, name="ref_unet_seq_256.pt", B=2, T=4, hw=(32, 16, 8), feat_seed=256256)
+    unet_seq(ref, wi, name="ref_unet_seq_256.pt", B=2, T=4, hw=(32, 16, 8), feat_seed=256256, sample_outs=True)

@@ -14,7 +14,9 @@ fp32 conv and the tcgen05 bf16 x bf16 -> fp32 conv then multiply identical numbe
 
 Weights are not stored (MBs): they are re-created from the recorded seed through the same constructor + the reference's
 `initialize_weights` (weight_initialization.py:8-56), which the product mirrors draw for draw; per-tensor checksums pin
-that.  Gradients are stored as norms + a 1-in-29 strided sample.
+that.  Inputs and upstream gradients are not stored either: they are the next draws of the same seeded generator, and
+their shapes and checksums are.  Gradients are stored as norms + a 1-in-29 strided sample, output tensors as norm, shape
+and a 1-in-7 strided sample (compact(), which keeps the file under 1 MB).
 """
 import os
 import sys
@@ -27,6 +29,8 @@ from oracle.ref_loader import load_reference  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
 STRIDE = 29
+OUT_STRIDE = 7
+INPUTS = ("x", "skip", "gy", "xs", "gh", "gc")
 
 
 def bf16r(t):
@@ -57,6 +61,32 @@ def checks(m):
 
 def grads(m):
     return {k: dict(norm=float(p.grad.double().norm()), sample=sample(p.grad)) for k, p in m.named_parameters()}
+
+
+def compact(fx):
+    """In place: every input / upstream gradient -> {shape, sum, abs} (the test draws it again from the generator, in the
+    order of INPUTS, and checks the sums), every other tensor of more than 256 elements -> {shape, norm, sample} with an
+    OUT_STRIDE strided sample of the flattened tensor."""
+    def inp(t):
+        assert torch.equal(bf16r(t.float()), t.float())        # bf16-representable by construction
+        t = t.double()
+        return dict(shape=tuple(t.shape), sum=float(t.sum()), abs=float(t.abs().sum()))
+
+    def out(t):
+        return dict(shape=tuple(t.shape), norm=float(t.double().norm()), sample=t.detach().float().flatten()[::OUT_STRIDE].clone())
+
+    fx["out_stride"] = OUT_STRIDE
+    for rec in fx.values():
+        if not isinstance(rec, dict):
+            continue
+        for k, v in rec.items():
+            if k in INPUTS:
+                rec[k] = [inp(t) for t in v] if isinstance(v, list) else inp(v)
+            elif isinstance(v, list) and all(torch.is_tensor(t) for t in v):
+                rec[k] = [out(t) for t in v]
+            elif torch.is_tensor(v) and v.numel() > 256:
+                rec[k] = out(v)
+    return fx
 
 
 def main():
@@ -125,15 +155,7 @@ def main():
     fx["convlstm"] = dict(seed=107, checks=ck, xs=[x.detach().clone() for x in xs], hs=[h.detach().clone() for h in hs],
                           c_last=hid[1].detach().clone(), gh=gh, gc=gc, gxs=[x.grad.clone() for x in xs], grads=grads(m))
 
-    # inputs / upstream gradients are bf16-representable by construction: store them as bf16 (half the bytes, lossless)
-    for rec in fx.values():
-        if isinstance(rec, dict):
-            for k in ("x", "gy", "skip", "gh", "gc"):
-                if k in rec:
-                    assert torch.equal(bf16r(rec[k]), rec[k])
-                    rec[k] = rec[k].to(torch.bfloat16)
-            if "xs" in rec:
-                rec["xs"] = [t.to(torch.bfloat16) for t in rec["xs"]]
+    compact(fx)
     path = os.path.join(OUT, "ref_blocks_path.pt")
     torch.save(fx, path)
     print("ref_blocks_path.pt", os.path.getsize(path))

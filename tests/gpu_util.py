@@ -15,6 +15,15 @@ def rel_err(a, b):
     return float((a - b).norm() / (b.norm() + 1e-30))
 
 
+def sampled_rel_err(got, ref, stride):
+    """rel_err against a fixture tensor stored as {shape, norm, sample} (every stride-th element of the flattened tensor):
+    the larger of the error at the stored positions and the error of the whole tensor's norm."""
+    got = got.detach().float().cpu()
+    assert tuple(got.shape) == tuple(ref["shape"]), (tuple(got.shape), ref["shape"])
+    en = abs(float(got.double().norm()) - ref["norm"]) / (ref["norm"] + 1e-30)
+    return max(rel_err(got.flatten()[::stride], ref["sample"]), en)
+
+
 def max_err(a, b):
     return float((a.double() - b.double()).abs().max())
 

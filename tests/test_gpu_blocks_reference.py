@@ -1,7 +1,7 @@
 """-m gpu: the CUDA blocks against the REAL reference classes, block by block (teacher-forced).
 
 Fixture: tests/golden/ref_blocks_path.pt, recorded by tests/golden/make_golden_path.py from the unmodified
-/root/reference/model.py classes at the channel counts TemporalUNet instantiates them with (model.py:104-119):
+reference model.py classes at the channel counts TemporalUNet instantiates them with (model.py:104-119):
 ConvBlock(144,128), ConvBlock(128,256,stride=2), DownBlock(128,256), UpBlock(256,128,128) with a same-size skip and
 with the bilinear skip-resize branch (model.py:43-44), ConvLSTM2d(128,128) over 3 steps.
 
@@ -13,13 +13,15 @@ multiply identical numbers.  Stated tolerances (rel = ||a-b|| / ||b||):
   * weight / BN-affine gradients (fp32 accumulators)  3e-3   dy operand rounding only
   * two-layer blocks (conv2 consumes bf16-rounded activations of conv1): 2x the above
 north_star: "rel 1e-3 in bf16 conv" -- met on the conv itself (1e-5); the 2e-3 lines are the bf16 storage rounding.
+Inputs are drawn again from the recorded seed (checksums pinned); outputs are compared at a 1-in-7 strided sample and by
+their norm over the whole tensor (sampled_rel_err).
 """
 import os
 
 import pytest
 import torch
 
-from tests.gpu_util import rel_err, setup_exact
+from tests.gpu_util import rel_err, sampled_rel_err, setup_exact
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -46,6 +48,15 @@ def _prepare(m, g):
                 mod.weight.copy_(torch.rand(mod.weight.shape, generator=g) * 0.8 + 0.8)
                 mod.bias.copy_(torch.rand(mod.bias.shape, generator=g) * 0.7 - 0.2)
     return m
+
+
+def _draw(g, spec):
+    """The next fixture input: drawn from the seeded generator as make_golden_path.py drew it, checked against the
+    recorded checksums."""
+    t = _bf16r(torch.randn(*spec["shape"], generator=g))
+    s, a = float(t.double().sum()), float(t.double().abs().sum())
+    assert abs(s - spec["sum"]) <= 1e-9 * spec["abs"] and abs(a - spec["abs"]) <= 1e-9 * spec["abs"], spec["shape"]
+    return t
 
 
 def _check_init(m, rec):
@@ -85,17 +96,19 @@ def test_convblock_vs_reference(fx, name):
     m = _prepare(M.ConvBlock(rec["ci"], rec["co"], stride=rec["stride"], neuron="silu"), g)
     _check_init(m, rec)
     m = m.to(DEV).train()
-    x = rec["x"].float().to(DEV).requires_grad_(True)
+    x = _draw(g, rec["x"]).to(DEV).requires_grad_(True)
+    gy = _draw(g, rec["gy"]).to(DEV)
+    so = fx["out_stride"]
     # the conv alone, fp32 out: identical bf16 operands -> summation order only
     st = store_for(m, DEV)
     st.refresh_operands()
     geom = 0 if rec["stride"] == 1 else 1
     cy = K.conv_fprop(geom, x.detach().permute(0, 2, 3, 1).to(torch.bfloat16).contiguous(), st.w_fprop(m.conv.weight), rec["co"])
-    e_conv = rel_err(cy.permute(0, 3, 1, 2).cpu(), rec["conv_y"])
+    e_conv = sampled_rel_err(cy.permute(0, 3, 1, 2), rec["conv_y"], so)
     y = m(x)
-    e_y = rel_err(y.detach().cpu(), rec["y_train"])
-    y.backward(rec["gy"].float().to(DEV))
-    e_gx = rel_err(x.grad.cpu(), rec["gx"])
+    e_y = sampled_rel_err(y, rec["y_train"], so)
+    y.backward(gy)
+    e_gx = sampled_rel_err(x.grad, rec["gx"], so)
     e_rm, e_rv = rel_err(m.bn.running_mean.cpu(), rec["running_mean"]), rel_err(m.bn.running_var.cpu(), rec["running_var"])
     print(f"\n{name}: conv {e_conv:.2e}  y {e_y:.2e}  gx {e_gx:.2e}  running mean/var {e_rm:.1e}/{e_rv:.1e}")
     assert e_conv < 1e-5 and e_y < 2e-3 and e_gx < 4e-3 and e_rm < 1e-5 and e_rv < 1e-5
@@ -103,7 +116,7 @@ def test_convblock_vs_reference(fx, name):
     m.eval()
     with torch.no_grad():
         ye = m(x.detach())
-    assert rel_err(ye.cpu(), rec["y_eval"]) < 2e-3
+    assert sampled_rel_err(ye, rec["y_eval"], so) < 2e-3
 
 
 def test_downblock_vs_reference(fx):
@@ -115,10 +128,12 @@ def test_downblock_vs_reference(fx):
     m = _prepare(M.DownBlock(128, 256, neuron="silu"), g)
     _check_init(m, rec)
     m = m.to(DEV).train()
-    x = rec["x"].float().to(DEV).requires_grad_(True)
+    x = _draw(g, rec["x"]).to(DEV).requires_grad_(True)
+    gy = _draw(g, rec["gy"]).to(DEV)
     y = m(x)
-    y.backward(rec["gy"].float().to(DEV))
-    e_y, e_gx = rel_err(y.detach().cpu(), rec["y"]), rel_err(x.grad.cpu(), rec["gx"])
+    y.backward(gy)
+    so = fx["out_stride"]
+    e_y, e_gx = sampled_rel_err(y, rec["y"], so), sampled_rel_err(x.grad, rec["gx"], so)
     print(f"\ndownblock: y {e_y:.2e}  gx {e_gx:.2e}")
     assert e_y < 4e-3 and e_gx < 8e-3
     _check_grads(m, rec, fx["stride"], 6e-3)
@@ -135,12 +150,14 @@ def test_upblock_vs_reference(fx, name):
     m = _prepare(M.UpBlock(256, 128, 128, neuron="silu"), g)
     _check_init(m, rec)
     m = m.to(DEV).train()
-    x = rec["x"].float().to(DEV).requires_grad_(True)
-    skip = rec["skip"].float().to(DEV).requires_grad_(True)
+    x = _draw(g, rec["x"]).to(DEV).requires_grad_(True)
+    skip = _draw(g, rec["skip"]).to(DEV).requires_grad_(True)
+    gy = _draw(g, rec["gy"]).to(DEV)
     y = m(x, skip)
-    assert tuple(y.shape) == tuple(rec["y"].shape)
-    y.backward(rec["gy"].float().to(DEV))
-    e_y, e_gx, e_gs = rel_err(y.detach().cpu(), rec["y"]), rel_err(x.grad.cpu(), rec["gx"]), rel_err(skip.grad.cpu(), rec["gskip"])
+    assert tuple(y.shape) == tuple(rec["y"]["shape"])
+    y.backward(gy)
+    so = fx["out_stride"]
+    e_y, e_gx, e_gs = sampled_rel_err(y, rec["y"], so), sampled_rel_err(x.grad, rec["gx"], so), sampled_rel_err(skip.grad, rec["gskip"], so)
     print(f"\n{name}: y {e_y:.2e}  gx {e_gx:.2e}  gskip {e_gs:.2e}")
     # the transposed conv's output and (resize branch) the interpolated skip are rounded to bf16 as conv1's operands
     assert e_y < 6e-3 and e_gx < 1e-2 and e_gs < 1e-2
@@ -185,15 +202,17 @@ def test_convlstm_vs_reference(fx):
     m = _prepare(M.ConvLSTM2d(128, 128), g)
     _check_init(m, rec)
     m = m.to(DEV)
-    xs = [x.float().to(DEV).requires_grad_(True) for x in rec["xs"]]
+    xs = [_draw(g, spec).to(DEV).requires_grad_(True) for spec in rec["xs"]]
+    gh, gc = _draw(g, rec["gh"]).to(DEV), _draw(g, rec["gc"]).to(DEV)
+    so = fx["out_stride"]
     hid, hs = None, []
     for x in xs:
         h, hid = m(x, hid)
         hs.append(h)
-    errs = [rel_err(h.detach().cpu(), r) for h, r in zip(hs, rec["hs"])]
-    e_c = rel_err(hid[1].detach().cpu(), rec["c_last"])
-    ((hs[-1] * rec["gh"].float().to(DEV)).sum() + (hid[1] * rec["gc"].float().to(DEV)).sum()).backward()
-    e_gx = [rel_err(x.grad.cpu(), r) for x, r in zip(xs, rec["gxs"])]
+    errs = [sampled_rel_err(h, r, so) for h, r in zip(hs, rec["hs"])]
+    e_c = sampled_rel_err(hid[1], rec["c_last"], so)
+    ((hs[-1] * gh).sum() + (hid[1] * gc).sum()).backward()
+    e_gx = [sampled_rel_err(x.grad, r, so) for x, r in zip(xs, rec["gxs"])]
     print(f"\nconvlstm: h {errs}  c {e_c:.2e}  gx {e_gx}")
     # step 1 has h = 0: identical operands -> 1e-5; later steps feed h back as a bf16-rounded conv operand (2^-9)
     assert errs[0] < 1e-5 and max(errs) < 2e-3 and e_c < 2e-3

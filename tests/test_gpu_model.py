@@ -16,7 +16,7 @@ import pytest
 import torch
 
 from oracle import snn_oracle as O
-from tests.gpu_util import rel_err, setup_exact
+from tests.gpu_util import rel_err, sampled_rel_err, setup_exact
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -72,7 +72,7 @@ def test_silu_unet_matches_reference_fixture(golden_dir):
     loss = sum((o ** 2).mean() for o in outs)
     loss.backward()
     for o, r in zip(outs, fx["outs"]):
-        assert rel_err(o.detach().cpu(), r) < 3e-2
+        assert sampled_rel_err(o, r, fx["out_stride"]) < 3e-2
     assert rel_err(hid[0].detach().cpu(), fx["h"]) < 3e-2 and rel_err(hid[1].detach().cpu(), fx["c"]) < 3e-2
     assert abs(float(loss) - fx["loss"]) < 1e-2 * fx["loss"]
     assert int(net.enc1.bn.num_batches_tracked) == fx["num_batches_tracked"]

@@ -308,3 +308,51 @@ def test_bench_comm_overlap_accounting():
     assert c["exposed_comm_ms_per_step"] == pytest.approx(0.035) and c["nccl_resident_ms_per_step"] == pytest.approx(0.075)
     assert c["nccl_kernels"]["ncclDevKernel_AllReduce_Sum_f32"]["launches_per_step"] == 1.0
     assert bench.comm_overlap(evs[:2], 1) is None
+
+
+@pytest.mark.parametrize("record", ["bench_final_default_n1.json", "bench_final_strip_n8.json"])
+def test_bench_result_line_stays_compact(record):
+    """bench.result_line on full records of this benchmark (one GPU: 21 KB with the 18-row LIF sweep and 40 shapes; eight
+    GPUs: 11.6 KB with the NCCL timeline): one strict-JSON line below RESULT_LINE_MAX that keeps the headline, the
+    roofline, the per-kernel table and the baselines."""
+    import json
+    import bench
+    path = os.path.join(bench.ROOT, "profiles", "r2", record)
+    rec = json.loads(open(path).read().strip().splitlines()[-1])
+    assert len(json.dumps(rec)) > bench.RESULT_LINE_MAX
+    line = bench.result_line(rec)
+    assert len(line.encode()) < bench.RESULT_LINE_MAX and "\n" not in line
+    d = json.loads(line)
+    assert d["value"] == pytest.approx(rec["value"], rel=1e-5) and d["steps"] == rec["steps"] and d["n_gpus"] == rec["n_gpus"]
+    assert d["roofline"]["kernel"] == rec["roofline"]["kernel"] and set(d["kernels"]) == set(rec["kernels"])
+    assert d["kernels_by_shape"] == rec["kernels_by_shape"][:8]
+    assert (d["comm_timeline"] is None) == (rec["comm_timeline"] is None)
+    if rec["lif_microbench"]:
+        assert d["cpu_baseline"]["cores"] == rec["cpu_baseline"]["cores"]
+        assert d["lif_microbench"]["fwd_frac_min"] == pytest.approx(rec["lif_microbench"]["fwd_frac_min"], rel=1e-5)
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.dump_outputs: float32 .npy files of the step's results; the parameters in declaration order, or a sample at
+    seeded positions (the same in every run) once there are more than DUMP_PARAM_SAMPLES of them."""
+    import numpy as np
+    import bench
+    torch.manual_seed(0)
+    m = torch.nn.Sequential(torch.nn.Linear(64, 32), torch.nn.Linear(32, 3))
+    flat = torch.cat([p.detach().reshape(-1) for p in m.parameters()]).numpy()
+    args = (torch.arange(3.0), torch.ones(3), torch.tensor([2.5]), m)
+    bench.dump_outputs(str(tmp_path / "all"), *args)
+    assert sorted(os.listdir(tmp_path / "all")) == ["grad_norm.npy", "loss.npy", "loss_items.npy", "params_sample.npy"]
+    for f in os.listdir(tmp_path / "all"):
+        assert np.load(tmp_path / "all" / f).dtype == np.float32
+    assert np.array_equal(np.load(tmp_path / "all" / "params_sample.npy"), flat)
+    assert np.array_equal(np.load(tmp_path / "all" / "loss.npy"), [0.0, 1.0, 2.0])
+    old = bench.DUMP_PARAM_SAMPLES
+    try:
+        bench.DUMP_PARAM_SAMPLES = 500
+        bench.dump_outputs(str(tmp_path / "s1"), *args)
+        bench.dump_outputs(str(tmp_path / "s2"), *args)
+    finally:
+        bench.DUMP_PARAM_SAMPLES = old
+    s1, s2 = np.load(tmp_path / "s1" / "params_sample.npy"), np.load(tmp_path / "s2" / "params_sample.npy")
+    assert s1.shape == (500,) and np.array_equal(s1, s2) and np.isin(s1, flat).all()
