@@ -236,6 +236,27 @@ int snn_nms(const float* pred, int B, int nc, int A, float conf_thres, float iou
             int max_det, int max_nms, float max_wh, unsigned long long* keys, long long keys_per_image,
             float* out, int* out_idx, int* counts, void* stream);
 
+/* ---- detection metrics: replaces ultralytics DetectionValidator / DetMetrics as called at eval_2.py:82-88 (mAP50,
+ *      mAP50-95, precision, recall).
+ *      snn_det_match, once per batch: rows fp32 [B][max_det][6] and counts int32 [B] = snn_nms output; gt_cls int64 [B][M],
+ *      gt_box fp32 [B][M][4] normalised (cx,cy,w,h), gt_valid uint8 [B][M] = the padded labels (M <= 2048); iou_thres
+ *      device fp32 [10].  Each kept row takes its same-class gt of highest IoU (box_iou, fp32; exact ties: the higher gt
+ *      index) and is a TP at threshold t when that IoU >= t and it is the lowest row claiming that gt.  Writes one record
+ *      per kept row at *cursor + sum(counts[<b]) -- rec_conf fp32, rec_cls int32, rec_tp uint16 (bit t = TP at
+ *      iou_thres[t]), rec_key int64 = (cls << 32) | (0x7FFFFFFF - float_bits(conf)) -- and advances *cursor (int64) by
+ *      sum(counts); ticket uint32[1] (zero-initialised once; left zeroed).  n_gt int64 [nc] += the gt class histogram;
+ *      err int32[1] += out-of-range gt / row classes and records past `capacity`.  No host synchronisation.
+ *      snn_det_metrics_finalize, once per evaluation: keys = rec_key[0..n) sorted ascending (stable), order = the record
+ *      index of each sorted key, rec_tp by record index.  out fp64 [8 + 11*nc] = {mp, mr, mAP50, mAP50-95, fitness,
+ *      number of target classes, F1 argmax, *err}, then ap [nc][10], then present [nc] (1 = class has gts); curves fp64
+ *      [2][nc][1000] = precision and recall curves at IoU 0.5 (scratch).  Keys >= (nc << 32) are ignored. ---- */
+int snn_det_match(const float* rows, const int* counts, int B, int max_det, const long long* gt_cls, const float* gt_box,
+                  const unsigned char* gt_valid, int M, float img_w, float img_h, const float* iou_thres, int nc,
+                  float* rec_conf, int* rec_cls, unsigned short* rec_tp, long long* rec_key, long long capacity,
+                  long long* cursor, unsigned int* ticket, long long* n_gt, int* err, void* stream);
+int snn_det_metrics_finalize(const long long* keys, const long long* order, const unsigned short* rec_tp, long long n,
+                             const long long* n_gt, int nc, const int* err, double* curves, double* out, void* stream);
+
 /* ---- detection-loss tail: replaces the per-anchor part of ultralytics v8DetectionLoss called at train.py:74
  *      (BCE class loss, CIoU box loss, DFL) given the assigner's targets.  N = B*A anchors (A = anchors per image,
  *      scale-major), distri fp32 [N][4*reg_max], scores / tscores fp32 [N][nc], anchors fp32 [A][2] (grid units),

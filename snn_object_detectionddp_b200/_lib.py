@@ -52,6 +52,8 @@ _SIGNATURES = {
     "snn_tal_assign": [_P, _P, _P, _P, _P, _P, _P, _F, _F, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P],
     "snn_detect_loss_bwd_rows": [_P, _P, _I, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _I, _P],
     "snn_nms": [_P, _I, _I, _I, _F, _F, _I, _I, _I, _I, _F, _P, _L, _P, _P, _P, _P],
+    "snn_det_match": [_P, _P, _I, _I, _P, _P, _P, _I, _F, _F, _P, _I, _P, _P, _P, _P, _L, _P, _P, _P, _P, _P],
+    "snn_det_metrics_finalize": [_P, _P, _P, _L, _P, _I, _P, _P, _P, _P],
     "snn_grad_sumsq": [_P, _L, _P, _I, _P],
     "snn_adamw_step": [_P, _P, _P, _P, _P, _L, _P, _P, _P, _P, _I, _I, _P],
 }

@@ -133,6 +133,12 @@ long long tal_workspace_bytes(int, int, int);
 int launch_tal_assign(const float*, const float*, const float*, const float*, const long long*, const float*, const uint8_t*, float,
                       float, int, int, int, int, int, void*, float*, float*, uint8_t*, float**, int*, cudaStream_t);
 
+int launch_det_match(const float*, const int*, int, int, const long long*, const float*, const unsigned char*, int, float, float,
+                     const float*, int, float*, int*, unsigned short*, long long*, long long, long long*, unsigned int*,
+                     long long*, int*, cudaStream_t);
+int launch_det_metrics_finalize(const long long*, const long long*, const unsigned short*, long long, const long long*, int,
+                                const int*, double*, double*, cudaStream_t);
+
 }  // namespace snn
 
 using namespace snn;
@@ -175,6 +181,17 @@ int snn_nms(const float* pred, int B, int nc, int A, float conf_thres, float iou
             int* out_idx, int* counts, void* stream) {
     return launch_nms(pred, B, nc, A, conf_thres, iou_thres, multi_label, agnostic, max_det, max_nms, max_wh, keys,
                       keys_per_image, out, out_idx, counts, ST);
+}
+int snn_det_match(const float* rows, const int* counts, int B, int max_det, const long long* gt_cls, const float* gt_box,
+                  const unsigned char* gt_valid, int M, float img_w, float img_h, const float* iou_thres, int nc,
+                  float* rec_conf, int* rec_cls, unsigned short* rec_tp, long long* rec_key, long long capacity,
+                  long long* cursor, unsigned int* ticket, long long* n_gt, int* err, void* stream) {
+    return launch_det_match(rows, counts, B, max_det, gt_cls, gt_box, gt_valid, M, img_w, img_h, iou_thres, nc, rec_conf, rec_cls,
+                            rec_tp, rec_key, capacity, cursor, ticket, n_gt, err, ST);
+}
+int snn_det_metrics_finalize(const long long* keys, const long long* order, const unsigned short* rec_tp, long long n,
+                             const long long* n_gt, int nc, const int* err, double* curves, double* out, void* stream) {
+    return launch_det_metrics_finalize(keys, order, rec_tp, n, n_gt, nc, err, curves, out, ST);
 }
 long long snn_bn_finalize_workspace_doubles(int T, int C, int groups_per_step) { return bn_finalize_workspace_doubles(T, C, groups_per_step); }
 int snn_bn_finalize_partials(const float* partials, double* sums, double* workspace, const float* gamma, const float* beta,

@@ -22,13 +22,19 @@ def decode_last_step(model, frames, hidden_state=None, return_state=False):
         det, hidden = model.forward_sequence(frames, hidden_state, return_state=return_state)
     finally:
         model.train(was_training)
+    return decode_head(model, det), hidden
+
+
+@torch.no_grad()
+def decode_head(model, det):
+    """Detect-head output of an eval-mode forward -> prediction [B, 4+nc, A] (xywh pixels + class scores)."""
     head = model.detection_head
     distri, scores = det.flat()
     from .head import make_anchors
     anchors, strides = make_anchors(det.shapes(), head.stride.tolist(), 0.5, device=distri.device)
     boxes, probs = K.detect_decode(distri.contiguous(), scores.contiguous(), anchors.contiguous(), strides.view(-1).contiguous(),
                                    xywh=True)
-    return torch.cat((boxes, probs), 2).permute(0, 2, 1).contiguous(), hidden
+    return torch.cat((boxes, probs), 2).permute(0, 2, 1).contiguous()
 
 
 @torch.no_grad()

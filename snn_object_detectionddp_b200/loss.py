@@ -141,6 +141,18 @@ def pad_targets(labels, batch_size, device=None, max_boxes=None):
     return cls, box, valid
 
 
+def batch_targets(batch, batch_size, device):
+    """The targets of a loss batch -- {'padded': pad_targets(...)} or the collate dict {'batch_idx', 'cls', 'bboxes'}
+    (train.py:68-72) -- as device tensors (cls long [B,M], xywh fp32 [B,M,4], valid bool [B,M])."""
+    if "padded" in batch:
+        cls, box, valid = (t.to(device, non_blocking=True) for t in batch["padded"])
+    else:
+        lab = torch.cat((batch["batch_idx"].view(-1, 1).float(), batch["cls"].view(-1, 1).float(),
+                         batch["bboxes"].view(-1, 4).float()), 1)
+        cls, box, valid = pad_targets(lab, batch_size, device)
+    return cls.long().contiguous(), box.float().contiguous(), valid.contiguous()
+
+
 class v8DetectionLoss:
     def __init__(self, model, tal_topk=10):
         m = model.model[-1]                       # the Detect module (reference model.py:195)
@@ -173,13 +185,7 @@ class v8DetectionLoss:
         return cat[..., :4 * self.reg_max].contiguous(), cat[..., 4 * self.reg_max:].contiguous(), [tuple(f.shape[2:]) for f in feats]
 
     def _labels(self, batch, B, dev):
-        if "padded" in batch:
-            cls, box, valid = (t.to(dev, non_blocking=True) for t in batch["padded"])
-        else:
-            lab = torch.cat((batch["batch_idx"].view(-1, 1).float(), batch["cls"].view(-1, 1).float(),
-                             batch["bboxes"].view(-1, 4).float()), 1)
-            cls, box, valid = pad_targets(lab, B, dev)
-        return cls.long().contiguous(), box.float().contiguous(), valid.contiguous()
+        return batch_targets(batch, B, dev)
 
     def __call__(self, preds, batch):
         from .head import HeadOut

@@ -107,8 +107,11 @@ def train_one_epoch(trainer, dataloader, sequence_length=None, writer=None, epoc
 
 
 @torch.no_grad()
-def validate_one_epoch(trainer, dataloader, sequence_length=None, writer=None, epoch=0, log_every=50, max_boxes=None):
-    """reference train.py:106-146: eval mode, state reset per window, loss on the last frame."""
+def validate_one_epoch(trainer, dataloader, sequence_length=None, writer=None, epoch=0, log_every=50, max_boxes=None,
+                       metrics=None):
+    """reference train.py:106-146: eval mode, state reset per window, loss on the last frame.  `metrics`: a
+    metrics.DetMetrics that also receives the detections of the same forwards (call its compute() afterwards)."""
+    det_metrics = metrics
     metrics = DeviceMetrics(trainer.device, log_every)
     n_batches = len(dataloader)
     for batch_idx, (image_tensor, labels_tensor) in enumerate(dataloader):
@@ -116,7 +119,7 @@ def validate_one_epoch(trainer, dataloader, sequence_length=None, writer=None, e
             image_tensor = image_tensor[:, :sequence_length]
         frames = image_tensor.to(trainer.device, non_blocking=True)
         batch = _batch_dict(trainer, labels_tensor, frames.shape[0], max_boxes)
-        items = trainer.validate_step(frames.contiguous(), batch)
+        items = trainer.validate_step(frames.contiguous(), batch, metrics=det_metrics)
         if metrics.update(items, epoch * n_batches + batch_idx):
             _log_batches(writer, metrics.flush(), False)
     _log_batches(writer, metrics.flush(), False)
@@ -124,10 +127,11 @@ def validate_one_epoch(trainer, dataloader, sequence_length=None, writer=None, e
 
 
 def train_loop(model, train_loader, val_loader, config, device, save_dir, process_group=None, writer=None, log_every=50, graphed=False,
-               max_boxes=None):
+               max_boxes=None, eval_map=False):
     """reference train.py:148-241: epochs of train + validation, `latest.pt` every epoch and `best.pt` on improvement (the
     reference's checkpoint dict, plus optimizer state), the reference's epoch-level TensorBoard tags.
-    Returns the Trainer (the reference returns None)."""
+    eval_map=True: the validation forwards also feed a DetMetrics, and metrics/{precision,recall,mAP50,mAP50-95}(B) are
+    logged every epoch.  Returns the Trainer (the reference returns None)."""
     from .trainer import Trainer
     if writer is None:
         try:
@@ -142,14 +146,25 @@ def train_loop(model, train_loader, val_loader, config, device, save_dir, proces
     seq_len = config["dataset"]["train"]["seq_len"]
     best_val_loss = float("inf")
     rank0 = (not torch.distributed.is_initialized()) or torch.distributed.get_rank() == 0
+    det_metrics = None
+    if eval_map:
+        from .metrics import KEYS, DetMetrics
+        det_metrics = DetMetrics(model.nc, trainer.device)
     for epoch in range(tc["epochs"]):
         sampler = getattr(train_loader, "sampler", None)
         if hasattr(sampler, "set_epoch"):
             sampler.set_epoch(epoch)
         train_loss, train_comps = train_one_epoch(trainer, train_loader, seq_len, writer=writer, epoch=epoch, log_every=log_every,
                                                   max_boxes=max_boxes, graphed=graphed)
+        if det_metrics is not None:
+            det_metrics.reset()
         val_loss, val_comps = validate_one_epoch(trainer, val_loader, seq_len, writer=writer, epoch=epoch, log_every=log_every,
-                                                 max_boxes=max_boxes)
+                                                 max_boxes=max_boxes, metrics=det_metrics)
+        if det_metrics is not None:
+            res = det_metrics.compute(_metrics_group(process_group))
+            if writer is not None and rank0:
+                for tag in KEYS[:4]:                        # metrics/{precision,recall,mAP50,mAP50-95}(B)
+                    writer.add_scalar(tag, res[tag], epoch)
         if rank0:
             os.makedirs(str(save_dir), exist_ok=True)
             trainer.save_checkpoint(os.path.join(str(save_dir), "latest.pt"), epoch=epoch, best_val_loss=best_val_loss)
@@ -164,6 +179,40 @@ def train_loop(model, train_loader, val_loader, config, device, save_dir, proces
             if rank0:
                 trainer.save_checkpoint(os.path.join(str(save_dir), "best.pt"), epoch=epoch, best_val_loss=best_val_loss)
     return trainer
+
+
+def _metrics_group(process_group):
+    """The group the detection records are gathered over: the trainer's, or the default one under torch.distributed."""
+    if process_group is not None:
+        return process_group
+    if torch.distributed.is_initialized() and torch.distributed.get_world_size() > 1:
+        return torch.distributed.group.WORLD
+    return None
+
+
+@torch.no_grad()
+def evaluate_model(model, dataloader, device, sequence_length=None, conf_thres=0.001, iou_thres=0.6, max_det=300,
+                   process_group=None):
+    """reference eval_2.py:20-130 as intended: every window of the loader through the eval-mode unroll (state reset per
+    window), decode and NMS at eval_2.py:108's settings (conf 0.001, iou 0.6, best class per anchor), matched against the
+    window's labels at IoU 0.50:0.05:0.95.  Returns DetMetrics.compute()'s dict: "metrics/precision(B)",
+    "metrics/recall(B)", "metrics/mAP50(B)", "metrics/mAP50-95(B)", "fitness", "ap", "ap_class_index".  Windows replay
+    from one CUDA graph (GraphedWindowDetector); the host reads the device once, at the end.  Under data parallelism
+    every rank evaluates its shard and gets the metric over all of them (see DetMetrics.compute)."""
+    from .infer import GraphedWindowDetector
+    from .loss import pad_targets
+    from .metrics import DetMetrics
+    device = torch.device(device)
+    model.to(device)
+    metrics = DetMetrics(model.nc, device)
+    detector = GraphedWindowDetector(model, conf_thres=conf_thres, iou_thres=iou_thres, multi_label=False, max_det=max_det)
+    for image_tensor, labels_tensor in dataloader:
+        if sequence_length is not None:
+            image_tensor = image_tensor[:, :sequence_length]
+        frames = image_tensor.to(device, non_blocking=True).contiguous()
+        rows, _, counts = detector(frames)
+        metrics.update(rows, counts, pad_targets(labels_tensor, frames.shape[0]), frames.shape[-2:])
+    return metrics.compute(_metrics_group(process_group))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -189,7 +238,8 @@ class ShardedSampler(torch.utils.data.Sampler):
     """Per-rank sampler (DistributedSampler semantics) for one process per GPU: every epoch a permutation seeded by
     (seed, epoch) -- identical on all ranks -- is padded (or truncated with drop_last) to a multiple of world_size and
     rank r takes elements r, r+world, ...  With world_size 1 and shuffle=True it is DataLoader(shuffle=True) with a
-    reproducible order (main.py:57-64)."""
+    reproducible order (main.py:57-64).  The padding repeats samples: a distributed evaluation (evaluate_model,
+    train_loop(eval_map=True)) counts the repeats like any other image, as with a stock DistributedSampler."""
 
     def __init__(self, data_source, rank=None, world_size=None, shuffle=True, seed=42, drop_last=False):
         if world_size is None:

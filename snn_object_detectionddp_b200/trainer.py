@@ -17,7 +17,7 @@ import torch.distributed as dist
 
 from . import kernels as K
 from .ddp import GradBucketer, broadcast_module_state
-from .loss import pad_targets, v8DetectionLoss
+from .loss import batch_targets, pad_targets, v8DetectionLoss
 from .params import store_for
 
 
@@ -160,15 +160,22 @@ class Trainer:
 
     # ------------------------------------------------------------------------------------------
     @torch.no_grad()
-    def validate_step(self, frames, batch):
+    def validate_step(self, frames, batch, metrics=None, conf_thres=0.001, iou_thres=0.6, max_det=300):
         """validate_one_epoch's inner step (reference train.py:106-131): eval mode (BatchNorm running statistics, state
-        reset per window), loss on the last frame, no gradient.  Returns loss.detach() [3] as a DEVICE tensor."""
+        reset per window), loss on the last frame, no gradient.  Returns loss.detach() [3] as a DEVICE tensor.
+        metrics: a metrics.DetMetrics -- the same forward is also decoded, put through NMS (eval_2.py:108 settings) and
+        matched against the batch's targets, without a host synchronisation."""
         model = self.model
         was_training = model.training
         model.eval()
         try:
             det, _ = model.forward_sequence(frames)
             _, items = self.loss_fn(det, batch)
+            if metrics is not None:
+                from .infer import decode_head
+                from .nms import non_max_suppression_padded
+                rows, _, counts = non_max_suppression_padded(decode_head(model, det), conf_thres, iou_thres, max_det=max_det)
+                metrics.update(rows, counts, batch_targets(batch, frames.shape[0], frames.device), frames.shape[-2:])
         finally:
             model.train(was_training)
         return items
