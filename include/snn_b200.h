@@ -139,6 +139,11 @@ int snn_bn_finalize(const double* sums, const float* gamma, const float* beta,
 int snn_bn_act_fwd(int act, const float* y, const float* scale, const float* shift, const float* v_init,
                    void* out_bf16, uint8_t* mask, float* v_final, int T, long long n_per_t, int C,
                    int ss_stride_t, float beta, float theta, void* stream);
+/* snn_bn_act_fwd (LIF only) that also ADDS per-timestep totals: spikes[t] += #{s=1}, steps[t] += n_per_t (uint64, exact).
+ * Outputs are bit-identical to snn_bn_act_fwd(ACT_LIF, ...); T <= 64. */
+int snn_bn_act_fwd_count(const float* y, const float* scale, const float* shift, const float* v_init, void* out_bf16,
+                         uint8_t* mask, float* v_final, unsigned long long* spikes, unsigned long long* steps,
+                         int T, long long n_per_t, int C, int ss_stride_t, float beta, float theta, void* stream);
 /* reverse-time surrogate-gradient scan. training!=0: writes gx fp32 [T][P][C] and red [T][2][C]
  * (sum gx, sum gx*xhat); training==0: writes dy bf16 = gx*scale directly. */
 int snn_bn_act_bwd(int act, int training, const float* y, const float* scale, const float* shift,

@@ -28,6 +28,7 @@ _SIGNATURES = {
     "snn_bn_stats": [_P, _P, _P, _I, _I, _I, _P],
     "snn_bn_finalize": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _F, _I, _P],
     "snn_bn_act_fwd": [_I, _P, _P, _P, _P, _P, _P, _P, _I, _L, _I, _I, _F, _F, _P],
+    "snn_bn_act_fwd_count": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _L, _I, _I, _F, _F, _P],
     "snn_bn_act_bwd": [_I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _F, _F, _P],
     "snn_bn_act_bwd2": [_I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _F, _F, _P],
     "snn_bn_bwd_dx": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P],

@@ -97,6 +97,8 @@ int launch_bn_finalize(const double*, const float*, const float*, float*, float*
                        float, float, int, cudaStream_t);
 int launch_bn_act_fwd(int, const float*, const float*, const float*, const float*, __nv_bfloat16*, uint8_t*, float*, int,
                       long long, int, int, float, float, cudaStream_t);
+int launch_bn_act_fwd_count(const float*, const float*, const float*, const float*, __nv_bfloat16*, uint8_t*, float*,
+                            unsigned long long*, unsigned long long*, int, long long, int, int, float, float, cudaStream_t);
 int launch_bn_act_bwd(int, int, const float*, const float*, const float*, const float*, const float*, const float*,
                       const __nv_bfloat16*, const float*, float*, __nv_bfloat16*, float*, float*, int, int, int, int, float,
                       float, float, cudaStream_t);
@@ -229,6 +231,12 @@ int snn_bn_act_fwd(int act, const float* y, const float* scale, const float* shi
                    void* stream) {
     return launch_bn_act_fwd(act, y, scale, shift, v_init, (__nv_bfloat16*)out, mask, v_final, T, n_per_t, C, ss_stride_t,
                              beta, theta, ST);
+}
+int snn_bn_act_fwd_count(const float* y, const float* scale, const float* shift, const float* v_init, void* out, uint8_t* mask,
+                         float* v_final, unsigned long long* spikes, unsigned long long* steps, int T, long long n_per_t, int C,
+                         int ss_stride_t, float beta, float theta, void* stream) {
+    return launch_bn_act_fwd_count(y, scale, shift, v_init, (__nv_bfloat16*)out, mask, v_final, spikes, steps, T, n_per_t, C,
+                                   ss_stride_t, beta, theta, ST);
 }
 int snn_bn_act_bwd(int act, int training, const float* y, const float* scale, const float* shift, const float* mean,
                    const float* invstd, const float* v_init, const void* gs, const float* gv_final, float* gx, void* dy,

@@ -250,21 +250,36 @@ __global__ void bn_finalize_kernel(const double* __restrict__ sums, const float*
 
 // ------------------------------------------------------------------------------------------
 // forward: x = y*scale + shift ; LIF scan over T (or SiLU) ; 8 channels / thread
+// COUNT (LIF only): also adds the number of spikes of each timestep to spikes[t] (popcount of the 8 spike bits, warp
+// reduce, block reduce in shared memory, one 64-bit integer atomic per block and timestep: exact, order-independent) and
+// n_per_t to steps[t] (block 0).  Out-of-range threads stay alive with no spikes so every lane reaches the warp reduce.
+// The counters are trailing parameters, so the uncounted instantiations compile to the code they had without them.
 // ------------------------------------------------------------------------------------------
-template <int ACT>
+constexpr int kCountMaxT = 64;    // timesteps one counted launch can tally (shared-memory slots)
+template <int ACT, bool COUNT>
 __global__ void __launch_bounds__(256) bn_act_fwd_kernel(const float* __restrict__ y, const float* __restrict__ scale,
                                                           const float* __restrict__ shift, const float* __restrict__ v_init,
                                                           __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ mask,
                                                           float* __restrict__ v_final, int T, long long n8, int C,
-                                                          int ss_stride_t, float beta, float theta) {
+                                                          int ss_stride_t, float beta, float theta,
+                                                          unsigned long long* __restrict__ spikes,
+                                                          unsigned long long* __restrict__ steps) {
     pdl_launch_dependents();
     pdl_wait();
     const long long idx = (long long)blockIdx.x * 256 + threadIdx.x;
-    if (idx >= n8) return;
-    const int c0 = (int)((idx * 8) % C);
+    if constexpr (!COUNT) {
+        if (idx >= n8) return;
+    }
+    const bool live = !COUNT || idx < n8;
+    __shared__ unsigned int s_cnt[COUNT ? kCountMaxT : 1];
+    if constexpr (COUNT) {
+        for (int t = threadIdx.x; t < T; t += 256) s_cnt[t] = 0u;
+        __syncthreads();
+    }
+    const int c0 = live ? (int)((idx * 8) % C) : 0;
     const size_t nt = (size_t)n8 * 8;
     float v[8];
-    if (ACT == ACT_LIF && v_init) {
+    if (ACT == ACT_LIF && v_init && live) {
         const float4 a = __ldg(reinterpret_cast<const float4*>(v_init) + idx * 2);
         const float4 b = __ldg(reinterpret_cast<const float4*>(v_init) + idx * 2 + 1);
         v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
@@ -274,41 +289,54 @@ __global__ void __launch_bounds__(256) bn_act_fwd_kernel(const float* __restrict
     }
 #pragma unroll 4
     for (int t = 0; t < T; ++t) {
-        const float4* yp = reinterpret_cast<const float4*>(y + (size_t)t * nt) + idx * 2;
-        const float4 ya = __ldcs(yp), yb = __ldcs(yp + 1);
-        const float4* sp = reinterpret_cast<const float4*>(scale + (size_t)t * ss_stride_t + c0);
-        const float4* hp = reinterpret_cast<const float4*>(shift + (size_t)t * ss_stride_t + c0);
-        const float4 sa = __ldg(sp), sb = __ldg(sp + 1), ha = __ldg(hp), hb = __ldg(hp + 1);
-        float x[8];
-        x[0] = __fadd_rn(__fmul_rn(ya.x, sa.x), ha.x); x[1] = __fadd_rn(__fmul_rn(ya.y, sa.y), ha.y);
-        x[2] = __fadd_rn(__fmul_rn(ya.z, sa.z), ha.z); x[3] = __fadd_rn(__fmul_rn(ya.w, sa.w), ha.w);
-        x[4] = __fadd_rn(__fmul_rn(yb.x, sb.x), hb.x); x[5] = __fadd_rn(__fmul_rn(yb.y, sb.y), hb.y);
-        x[6] = __fadd_rn(__fmul_rn(yb.z, sb.z), hb.z); x[7] = __fadd_rn(__fmul_rn(yb.w, sb.w), hb.w);
-        float o[8];
         uint32_t bits = 0;
-        if (ACT == ACT_LIF) {
+        if (live) {
+            const float4* yp = reinterpret_cast<const float4*>(y + (size_t)t * nt) + idx * 2;
+            const float4 ya = __ldcs(yp), yb = __ldcs(yp + 1);
+            const float4* sp = reinterpret_cast<const float4*>(scale + (size_t)t * ss_stride_t + c0);
+            const float4* hp = reinterpret_cast<const float4*>(shift + (size_t)t * ss_stride_t + c0);
+            const float4 sa = __ldg(sp), sb = __ldg(sp + 1), ha = __ldg(hp), hb = __ldg(hp + 1);
+            float x[8];
+            x[0] = __fadd_rn(__fmul_rn(ya.x, sa.x), ha.x); x[1] = __fadd_rn(__fmul_rn(ya.y, sa.y), ha.y);
+            x[2] = __fadd_rn(__fmul_rn(ya.z, sa.z), ha.z); x[3] = __fadd_rn(__fmul_rn(ya.w, sa.w), ha.w);
+            x[4] = __fadd_rn(__fmul_rn(yb.x, sb.x), hb.x); x[5] = __fadd_rn(__fmul_rn(yb.y, sb.y), hb.y);
+            x[6] = __fadd_rn(__fmul_rn(yb.z, sb.z), hb.z); x[7] = __fadd_rn(__fmul_rn(yb.w, sb.w), hb.w);
+            float o[8];
+            if (ACT == ACT_LIF) {
 #pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const float u = __fadd_rn(__fmul_rn(beta, v[i]), x[i]);
-                const bool s = u >= theta;
-                v[i] = s ? 0.f : u;
-                o[i] = s ? 1.f : 0.f;
-                bits |= (s ? 1u : 0u) << i;
+                for (int i = 0; i < 8; ++i) {
+                    const float u = __fadd_rn(__fmul_rn(beta, v[i]), x[i]);
+                    const bool s = u >= theta;
+                    v[i] = s ? 0.f : u;
+                    o[i] = s ? 1.f : 0.f;
+                    bits |= (s ? 1u : 0u) << i;
+                }
+            } else {
+#pragma unroll
+                for (int i = 0; i < 8; ++i) o[i] = x[i] / (1.f + __expf(-x[i]));
             }
-        } else {
-#pragma unroll
-            for (int i = 0; i < 8; ++i) o[i] = x[i] / (1.f + __expf(-x[i]));
+            uint4 pk;
+            pk.x = pack_bf16x2(o[0], o[1]); pk.y = pack_bf16x2(o[2], o[3]);
+            pk.z = pack_bf16x2(o[4], o[5]); pk.w = pack_bf16x2(o[6], o[7]);
+            *(reinterpret_cast<uint4*>(out + (size_t)t * nt) + idx) = pk;
+            if (ACT == ACT_LIF && mask) mask[(size_t)t * n8 + idx] = (uint8_t)bits;
         }
-        uint4 pk;
-        pk.x = pack_bf16x2(o[0], o[1]); pk.y = pack_bf16x2(o[2], o[3]);
-        pk.z = pack_bf16x2(o[4], o[5]); pk.w = pack_bf16x2(o[6], o[7]);
-        *(reinterpret_cast<uint4*>(out + (size_t)t * nt) + idx) = pk;
-        if (ACT == ACT_LIF && mask) mask[(size_t)t * n8 + idx] = (uint8_t)bits;
+        if constexpr (COUNT) {
+            const unsigned int n = __reduce_add_sync(0xffffffffu, (unsigned int)__popc(bits));
+            if ((threadIdx.x & 31) == 0 && n) atomicAdd(&s_cnt[t], n);
+        }
     }
-    if (ACT == ACT_LIF && v_final) {
+    if (ACT == ACT_LIF && v_final && live) {
         float4* vp = reinterpret_cast<float4*>(v_final) + idx * 2;
         vp[0] = make_float4(v[0], v[1], v[2], v[3]);
         vp[1] = make_float4(v[4], v[5], v[6], v[7]);
+    }
+    if constexpr (COUNT) {
+        __syncthreads();
+        for (int t = threadIdx.x; t < T; t += 256) {
+            if (s_cnt[t]) atomicAdd(spikes + t, (unsigned long long)s_cnt[t]);
+            if (blockIdx.x == 0) atomicAdd(steps + t, (unsigned long long)(n8 * 8));
+        }
     }
 }
 
@@ -1128,12 +1156,26 @@ int launch_bn_act_fwd(int act, const float* y, const float* scale, const float* 
     const long long n8 = n_per_t / 8;
     const unsigned blocks = (unsigned)((n8 + 255) / 256);
     if (act == ACT_LIF)
-        launch_pdl(bn_act_fwd_kernel<ACT_LIF>, dim3(blocks), dim3(256), 0, st, y, scale, shift, v_init, out, mask, v_final, T, n8, C,
-                                                           ss_stride_t, beta, theta);
+        launch_pdl(bn_act_fwd_kernel<ACT_LIF, false>, dim3(blocks), dim3(256), 0, st, y, scale, shift, v_init, out, mask, v_final, T,
+                   n8, C, ss_stride_t, beta, theta, (unsigned long long*)nullptr, (unsigned long long*)nullptr);
     else
-        launch_pdl(bn_act_fwd_kernel<ACT_SILU>, dim3(blocks), dim3(256), 0, st, y, scale, shift, v_init, out, mask, v_final, T, n8, C,
-                                                            ss_stride_t, beta, theta);
+        launch_pdl(bn_act_fwd_kernel<ACT_SILU, false>, dim3(blocks), dim3(256), 0, st, y, scale, shift, v_init, out, mask, v_final, T,
+                   n8, C, ss_stride_t, beta, theta, (unsigned long long*)nullptr, (unsigned long long*)nullptr);
     return check_cuda(cudaGetLastError(), "bn_act_fwd_kernel");
+}
+
+int launch_bn_act_fwd_count(const float* y, const float* scale, const float* shift, const float* v_init, __nv_bfloat16* out,
+                            uint8_t* mask, float* v_final, unsigned long long* spikes, unsigned long long* steps, int T,
+                            long long n_per_t, int C, int ss_stride_t, float beta, float theta, cudaStream_t st) {
+    SNN_REQUIRE(C % 8 == 0, "bn_act_fwd_count: C=%d must be a multiple of 8", C);
+    SNN_REQUIRE(n_per_t % C == 0, "bn_act_fwd_count: n_per_t not a multiple of C");
+    SNN_REQUIRE(T >= 1 && T <= kCountMaxT, "bn_act_fwd_count: T=%d must be in [1,%d]", T, kCountMaxT);
+    SNN_REQUIRE(spikes != nullptr && steps != nullptr, "bn_act_fwd_count: spikes and steps counters are required");
+    const long long n8 = n_per_t / 8;
+    const unsigned blocks = (unsigned)((n8 + 255) / 256);
+    launch_pdl(bn_act_fwd_kernel<ACT_LIF, true>, dim3(blocks), dim3(256), 0, st, y, scale, shift, v_init, out, mask, v_final, T, n8,
+               C, ss_stride_t, beta, theta, spikes, steps);
+    return check_cuda(cudaGetLastError(), "bn_act_fwd_kernel<LIF, count>");
 }
 
 template <int ACT, int TMAX, bool TRAIN>

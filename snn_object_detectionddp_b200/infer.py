@@ -80,10 +80,14 @@ class GraphedWindowDetector:
 
     @torch.no_grad()
     def __call__(self, frames):
-        key = (tuple(frames.shape), frames.dtype, frames.device)
+        stats = getattr(self.model, "spike_stats", None)
+        key = (tuple(frames.shape), frames.dtype, frames.device, stats)     # holds the stats: its counters outlive the graph
         if self._graph is None or key != self._key:
+            saved = None if stats is None else stats.counts.clone()
             for _ in range(self.warmup):
                 detect_sequence(self.model, frames, padded=True, **self.kw)
+            if saved is not None:
+                stats.counts.copy_(saved)          # the warm-up windows are not part of what the caller counts
             self._in = frames.clone()
             torch.cuda.synchronize()
             g = torch.cuda.CUDAGraph()

@@ -201,9 +201,14 @@ def bn_finalize(sums, gamma, beta, running_mean, running_var, T, C, P, eps, mome
     return scale, shift, mean, invstd
 
 
-def bn_act_fwd(act, y, scale, shift, T, v_init=None, want_mask=True, want_v_final=False, beta=0.5, theta=1.0):
-    """Fused BN affine + LIF scan over T (or SiLU).  y fp32 [T*B,H,W,C] -> bf16 same shape (+mask, +v_final)."""
-    require_cuda(y, scale, shift, v_init)
+def bn_act_fwd(act, y, scale, shift, T, v_init=None, want_mask=True, want_v_final=False, beta=0.5, theta=1.0,
+               spike_counts=None):
+    """Fused BN affine + LIF scan over T (or SiLU).  y fp32 [T*B,H,W,C] -> bf16 same shape (+mask, +v_final).
+    spike_counts: (spikes, steps) int64 device views of >= T elements (LIF only); the launch adds the number of spikes
+    of timestep t to spikes[t] and the number of neurons per timestep to steps[t].  Outputs are unchanged."""
+    if spike_counts is not None and act != ACT_LIF:
+        raise _lib.SnnKernelError("bn_act_fwd: spike counting needs the LIF neuron")
+    require_cuda(y, scale, shift, v_init, *(spike_counts or ()))
     c = y.shape[-1]
     n_per_t = y.numel() // T
     out = torch.empty(y.shape, device=y.device, dtype=torch.bfloat16)
@@ -217,6 +222,15 @@ def bn_act_fwd(act, y, scale, shift, T, v_init=None, want_mask=True, want_v_fina
     # algorithmic bytes per neuron-timestep (SURVEY.md 8d): 4 (y fp32) + 2 (spike bf16) + 1/8 (packed mask)
     nbytes = y.numel() * (6.0 + (0.125 if mask is not None else 0.0))
     nbytes += (0 if v_init is None else 4.0 * n_per_t) + (0 if v_final is None else 4.0 * n_per_t)
+    if spike_counts is not None:
+        spikes, steps = spike_counts
+        for t in (spikes, steps):
+            if t.dtype != torch.int64 or not t.is_contiguous() or t.numel() < T:
+                raise ValueError(f"spike_counts: contiguous int64 views of >= T={T} elements required, got {t.dtype} "
+                                 f"{tuple(t.shape)} contiguous={t.is_contiguous()}")
+        call("snn_bn_act_fwd_count", ptr(y), ptr(scale), ptr(shift), ptr(v_init), ptr(out), ptr(mask), ptr(v_final), ptr(spikes),
+             ptr(steps), T, n_per_t, c, ss, float(beta), float(theta), stream_ptr(), work=("byte", nbytes, f"T{T} n{n_per_t} C{c}"))
+        return out, mask, v_final
     call("snn_bn_act_fwd", act, ptr(y), ptr(scale), ptr(shift), ptr(v_init), ptr(out), ptr(mask), ptr(v_final), T, n_per_t,
          c, ss, float(beta), float(theta), stream_ptr(), work=("byte", nbytes, f"T{T} n{n_per_t} C{c}"))
     return out, mask, v_final

@@ -40,6 +40,7 @@ class RunCtx:
         # BatchNorm running statistics advance per frame as in the reference -- but skip the all-zero backward of the
         # dead frames.  None = every timestep is live.
         self.live_T = live_T
+        self.spike_stats = None     # spikes.SpikeStats the LIF ConvBlocks count into (None: uncounted launches)
 
 
 def _to_nhwc_bf16(x):
@@ -95,6 +96,8 @@ class ConvBlock(nn.Module):
             cfg["dead_grad_unread"] = getattr(rc, "dead_grad_unread", False)
         if slot_x0 is not None:
             cfg["slot_x0"] = slot_x0          # (GradSlot, 'first' | 'last'): see ops.GradSlot
+        if rc.spike_stats is not None and self.neuron.kind == "lif":
+            cfg["spike_counts"] = rc.spike_stats.layer_counts(self._snn_name, rc.T)
         if self.geom == GEOM_3x3_S2 and ((x0.shape[1] | x0.shape[2]) & 1):
             # odd H or W (e.g. the 15x20 P5 level of a 480x640 frame): zero-pad to even -- the extra row / column is exactly
             # the conv's own padding, so Ho = ceil(H/2) and the values equal nn.Conv2d(k3, s2, p1) on the odd-sized map
@@ -255,6 +258,46 @@ class TemporalUNet(nn.Module):
         o3 = out_conv(self.out_p3, d3, None)
         return (o3, o4, o5), (new_lstm, nm)
 
+    def spike_fanout(self, feature_hw):
+        """{LIF ConvBlock name: F}, F = multiply-accumulates one element of that block's spike output drives, summed over the
+        convs that consume it AS SPIKES (borders ignored: the per-element share of the dense MACs).  feature_hw = the (H, W)
+        of p3, p4, p5.  Mirrors forward_seq's wiring: the zero pad in front of a stride-2 conv on an odd map adds no spikes
+        (its conv still counts); a skip that UpBlock resizes bilinearly is no longer binary (its conv1 K-slice does not
+        count); the ConvLSTM h, the transposed-conv outputs and the extractor features are not spikes."""
+        if self.neuron.kind != "lif":
+            return {}
+        half = lambda hw: ((hw[0] + 1) // 2, (hw[1] + 1) // 2)
+        hw3, hw4, hw5 = (tuple(int(v) for v in hw) for hw in feature_hw)
+        hw_b = half(hw5)                                   # down3 output = ConvLSTM / bottleneck map
+        hw_u1 = (2 * hw_b[0], 2 * hw_b[1])
+        hw_u2 = (2 * hw_u1[0], 2 * hw_u1[1])
+        hw_u3 = (2 * hw_u2[0], 2 * hw_u2[1])
+        f = {}
+
+        def edge(src, consumer):
+            f[src] = f.get(src, 0.0) + _fanout(consumer)
+
+        edge("enc1", self.down1.conv1.conv)
+        edge("down1.conv1", self.down1.conv2.conv)
+        edge("down1.conv2", self.enc2.conv)
+        edge("enc2", self.down2.conv1.conv)
+        edge("down2.conv1", self.down2.conv2.conv)
+        edge("down2.conv2", self.enc3.conv)
+        edge("enc3", self.down3.conv1.conv)
+        edge("down3.conv1", self.down3.conv2.conv)
+        edge("down3.conv2", self.lstm.conv)                # the W_x K-slice of the gate conv
+        edge("bottleneck_conv", self.up1.up)
+        for up, skip, hw_skip, hw_up, out_conv in ((self.up1, "enc3", hw5, hw_u1, self.out_p5),
+                                                   (self.up2, "enc2", hw4, hw_u2, self.out_p4),
+                                                   (self.up3, "enc1", hw3, hw_u3, self.out_p3)):
+            if hw_skip == hw_up:
+                edge(skip, up.conv1.conv)
+            edge(up.conv1._snn_name, up.conv2.conv)
+            edge(up.conv2._snn_name, out_conv)
+        edge("up1.conv2", self.up2.up)
+        edge("up2.conv2", self.up3.up)
+        return f
+
     def forward(self, features, hidden_state=None):
         """Drop-in: features = 3 NCHW fp32 maps; hidden_state = None | (h, c) | (h, c, membranes)."""
         p3 = features[0]
@@ -264,6 +307,16 @@ class TemporalUNet(nn.Module):
         rc = RunCtx(st, 1, want_state=True, fp32_outputs=True)
         outs, new_state = self.forward_seq(rc, tuple(_to_nhwc_bf16(f) for f in features), state)
         return tuple(o.permute(0, 3, 1, 2) for o in outs), _pack_hidden(new_state, self.neuron.kind)
+
+
+def _fanout(conv):
+    """Multiply-accumulates one input element of `conv` drives (borders ignored): Cout/groups * kh * kw / (sh * sw) for a
+    Conv2d, Cout/groups * kh * kw for a ConvTranspose2d (every input pixel feeds each tap once)."""
+    kh, kw = conv.kernel_size
+    n = conv.out_channels // conv.groups * kh * kw
+    if isinstance(conv, nn.ConvTranspose2d):
+        return float(n)
+    return n / (conv.stride[0] * conv.stride[1])
 
 
 def _unpack_hidden(hidden_state):
@@ -381,6 +434,16 @@ class YOLOFeatureExtractor(nn.Module):
                 K.conv_fprop(GEOM_1x1, f4, self.w_p4, self.OUT, out_dtype=bf),
                 K.conv_fprop(GEOM_1x1, f5, self.w_p5, self.OUT, out_dtype=bf))
 
+    @staticmethod
+    def feature_hw(H, W):
+        """(H, W) of p3, p4, p5 for an H x W frame: stride 8, 16, 32 with every stride-2 stage rounding up."""
+        hw, out = (int(H), int(W)), []
+        for k in range(5):
+            hw = ((hw[0] + 1) // 2, (hw[1] + 1) // 2)
+            if k >= 2:
+                out.append(hw)
+        return out
+
     def forward(self, x):
         if self.backend == "ultralytics":      # reference model.py:88-91, verbatim semantics
             with torch.no_grad():
@@ -415,6 +478,16 @@ class YOLOTemporalUNet(nn.Module):
         self.register_buffer("strides", strides, persistent=False)
         self.model = nn.ModuleList([self.detection_head])
         self.skip_dead_backward = True      # see RunCtx.live_T (False: run the all-zero backward of the dead frames too)
+        # spikes.SpikeStats: while set, every forward / forward_sequence counts the LIF layers' spikes into it (a plain
+        # attribute: never in state_dict; captured CUDA graphs key on it, see Trainer.train_step_graphed)
+        self.spike_stats = None
+
+    def _spike_stats_for(self, frames, T):
+        """The attached SpikeStats, checked against this forward (T, device, fan-out table) before anything launches."""
+        stats = getattr(self, "spike_stats", None)       # None also for a model pickled before the attribute existed
+        if stats is not None:
+            stats.begin_forward(self.temporal_unet, T, self.feature_extractor.feature_hw(*frames.shape[-2:]), frames.device)
+        return stats
 
     # ---- fused sequence path -------------------------------------------------------------
     def forward_sequence(self, frames, hidden_state=None, return_state=False, all_steps=False, record=None):
@@ -422,10 +495,12 @@ class YOLOTemporalUNet(nn.Module):
         `hidden` is None unless return_state (final LSTM state + LIF membranes, for streaming inference).
         `record`: optional dict that receives every ConvBlock's output (spikes) by module name (flip-rate reports)."""
         B, T = frames.shape[0], frames.shape[1]
+        stats = self._spike_stats_for(frames, T)
         st = store_for(self, frames.device)
         st.refresh_operands()
         feats = self.feature_extractor.forward_seq(frames, B, T)
         rc = RunCtx(st, T, want_state=return_state, live_T=None if (all_steps or not self.skip_dead_backward) else 1)
+        rc.spike_stats = stats
         # the head's inputs are produced by the U-Net output convs, which slice the dead frames' gradient away themselves:
         # head-internal gradients of the dead frames are never read and need no zero fill
         rc.dead_grad_unread = rc.live_T is not None
@@ -438,10 +513,12 @@ class YOLOTemporalUNet(nn.Module):
     # ---- drop-in per-frame path (train.py:66, visualize.py:71) ----------------------------
     def forward(self, x, hidden_state=None):
         B = x.shape[0]
+        stats = self._spike_stats_for(x, 1)
         st = store_for(self, x.device)
         st.refresh_operands()
         feats = self.feature_extractor.forward_seq(x, B, 1)
         rc = RunCtx(st, 1, want_state=True)
+        rc.spike_stats = stats
         outs, new_state = self.temporal_unet.forward_seq(rc, feats, _unpack_hidden(hidden_state))
         det = self.detection_head.forward_seq(rc, outs, B, last_only=True)
         return det.as_reference(self.detection_head), _pack_hidden(new_state, self.temporal_unet.neuron.kind)

@@ -94,7 +94,7 @@ class ConvBNActFn(Function):
         want_state = cfg.get("want_state", False) and neuron.kind == "lif"
         out, mask, v_final = K.bn_act_fwd(neuron.act, y, scale, shift, T, v_init=v_init,
                                           want_mask=cfg.get("want_mask", False), want_v_final=want_state,
-                                          beta=neuron.beta, theta=neuron.v_th)
+                                          beta=neuron.beta, theta=neuron.v_th, spike_counts=cfg.get("spike_counts"))
         ctx.cfg = cfg
         ctx.has_x1 = x1 is not None
         ctx.has_v = v_init is not None

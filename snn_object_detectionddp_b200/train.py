@@ -127,11 +127,15 @@ def validate_one_epoch(trainer, dataloader, sequence_length=None, writer=None, e
 
 
 def train_loop(model, train_loader, val_loader, config, device, save_dir, process_group=None, writer=None, log_every=50, graphed=False,
-               max_boxes=None, eval_map=False):
+               max_boxes=None, eval_map=False, spike_stats=False):
     """reference train.py:148-241: epochs of train + validation, `latest.pt` every epoch and `best.pt` on improvement (the
     reference's checkpoint dict, plus optimizer state), the reference's epoch-level TensorBoard tags.
     eval_map=True: the validation forwards also feed a DetMetrics, and metrics/{precision,recall,mAP50,mAP50-95}(B) are
-    logged every epoch.  Returns the Trainer (the reference returns None)."""
+    logged every epoch.
+    spike_stats=True: one spikes.SpikeStats counts every forward of the loop; after each phase of an epoch it is read and
+    reset, and Spikes/{train,val}_rate, Spikes/{train,val}_synops_fraction and the per-layer validation rates
+    (Spikes_Val_Rate) are logged.  The model's previous `spike_stats` is restored on return.
+    Returns the Trainer (the reference returns None)."""
     from .trainer import Trainer
     if writer is None:
         try:
@@ -144,41 +148,68 @@ def train_loop(model, train_loader, val_loader, config, device, save_dir, proces
     trainer = Trainer(model, max_lr=tc["learning_rate"], weight_decay=tc["weight_decay"], total_steps=max(1, total_steps),
                       device=device, process_group=process_group)
     seq_len = config["dataset"]["train"]["seq_len"]
-    best_val_loss = float("inf")
     rank0 = (not torch.distributed.is_initialized()) or torch.distributed.get_rank() == 0
     det_metrics = None
     if eval_map:
         from .metrics import KEYS, DetMetrics
         det_metrics = DetMetrics(model.nc, trainer.device)
-    for epoch in range(tc["epochs"]):
-        sampler = getattr(train_loader, "sampler", None)
-        if hasattr(sampler, "set_epoch"):
-            sampler.set_epoch(epoch)
-        train_loss, train_comps = train_one_epoch(trainer, train_loader, seq_len, writer=writer, epoch=epoch, log_every=log_every,
-                                                  max_boxes=max_boxes, graphed=graphed)
-        if det_metrics is not None:
-            det_metrics.reset()
-        val_loss, val_comps = validate_one_epoch(trainer, val_loader, seq_len, writer=writer, epoch=epoch, log_every=log_every,
-                                                 max_boxes=max_boxes, metrics=det_metrics)
-        if det_metrics is not None:
-            res = det_metrics.compute(_metrics_group(process_group))
-            if writer is not None and rank0:
-                for tag in KEYS[:4]:                        # metrics/{precision,recall,mAP50,mAP50-95}(B)
-                    writer.add_scalar(tag, res[tag], epoch)
-        if rank0:
-            os.makedirs(str(save_dir), exist_ok=True)
-            trainer.save_checkpoint(os.path.join(str(save_dir), "latest.pt"), epoch=epoch, best_val_loss=best_val_loss)
-        if writer is not None and rank0:
-            writer.add_scalar("Loss/train", train_loss, epoch)
-            writer.add_scalar("Loss/val", val_loss, epoch)
-            writer.add_scalar("LearningRate", trainer.lr(), epoch)
-            writer.add_scalars("Train_Loss_Components", {k: float(v) for k, v in zip(COMPONENTS, train_comps)}, epoch)
-            writer.add_scalars("Val_Loss_Components", {k: float(v) for k, v in zip(COMPONENTS, val_comps)}, epoch)
-        if val_loss < best_val_loss:
-            best_val_loss = val_loss
+    prev_stats, stats = getattr(model, "spike_stats", None), None
+    if spike_stats:
+        from .spikes import MAX_T, SpikeStats
+        stats = SpikeStats(model, max_T=MAX_T)       # one buffer for both phases: the training graph is captured once
+        model.spike_stats = stats
+    log = writer is not None and rank0
+    best_val_loss = float("inf")
+    try:
+        for epoch in range(tc["epochs"]):
+            sampler = getattr(train_loader, "sampler", None)
+            if hasattr(sampler, "set_epoch"):
+                sampler.set_epoch(epoch)
+            train_loss, train_comps = train_one_epoch(trainer, train_loader, seq_len, writer=writer, epoch=epoch, log_every=log_every,
+                                                      max_boxes=max_boxes, graphed=graphed)
+            if stats is not None:
+                res = _spike_results(stats, process_group)
+                if log:
+                    writer.add_scalar("Spikes/train_rate", res["spikes/rate"], epoch)
+                    writer.add_scalar("Spikes/train_synops_fraction", res["spikes/synops_fraction"], epoch)
+            if det_metrics is not None:
+                det_metrics.reset()
+            val_loss, val_comps = validate_one_epoch(trainer, val_loader, seq_len, writer=writer, epoch=epoch, log_every=log_every,
+                                                     max_boxes=max_boxes, metrics=det_metrics)
+            if stats is not None:
+                res = _spike_results(stats, process_group)
+                if log:
+                    writer.add_scalar("Spikes/val_rate", res["spikes/rate"], epoch)
+                    writer.add_scalar("Spikes/val_synops_fraction", res["spikes/synops_fraction"], epoch)
+                    writer.add_scalars("Spikes_Val_Rate", {n: res["spikes/rate/" + n] for n in stats.layers}, epoch)
+            if det_metrics is not None:
+                res = det_metrics.compute(_metrics_group(process_group))
+                if log:
+                    for tag in KEYS[:4]:                        # metrics/{precision,recall,mAP50,mAP50-95}(B)
+                        writer.add_scalar(tag, res[tag], epoch)
             if rank0:
-                trainer.save_checkpoint(os.path.join(str(save_dir), "best.pt"), epoch=epoch, best_val_loss=best_val_loss)
+                os.makedirs(str(save_dir), exist_ok=True)
+                trainer.save_checkpoint(os.path.join(str(save_dir), "latest.pt"), epoch=epoch, best_val_loss=best_val_loss)
+            if writer is not None and rank0:
+                writer.add_scalar("Loss/train", train_loss, epoch)
+                writer.add_scalar("Loss/val", val_loss, epoch)
+                writer.add_scalar("LearningRate", trainer.lr(), epoch)
+                writer.add_scalars("Train_Loss_Components", {k: float(v) for k, v in zip(COMPONENTS, train_comps)}, epoch)
+                writer.add_scalars("Val_Loss_Components", {k: float(v) for k, v in zip(COMPONENTS, val_comps)}, epoch)
+            if val_loss < best_val_loss:
+                best_val_loss = val_loss
+                if rank0:
+                    trainer.save_checkpoint(os.path.join(str(save_dir), "best.pt"), epoch=epoch, best_val_loss=best_val_loss)
+    finally:
+        model.spike_stats = prev_stats
     return trainer
+
+
+def _spike_results(stats, process_group):
+    """compute() + reset() of the loop's SpikeStats (all ranks take part in the all_reduce)."""
+    res = stats.compute(_metrics_group(process_group))
+    stats.reset()
+    return res
 
 
 def _metrics_group(process_group):
@@ -192,13 +223,15 @@ def _metrics_group(process_group):
 
 @torch.no_grad()
 def evaluate_model(model, dataloader, device, sequence_length=None, conf_thres=0.001, iou_thres=0.6, max_det=300,
-                   process_group=None):
+                   process_group=None, spike_stats=False):
     """reference eval_2.py:20-130 as intended: every window of the loader through the eval-mode unroll (state reset per
     window), decode and NMS at eval_2.py:108's settings (conf 0.001, iou 0.6, best class per anchor), matched against the
     window's labels at IoU 0.50:0.05:0.95.  Returns DetMetrics.compute()'s dict: "metrics/precision(B)",
     "metrics/recall(B)", "metrics/mAP50(B)", "metrics/mAP50-95(B)", "fitness", "ap", "ap_class_index".  Windows replay
     from one CUDA graph (GraphedWindowDetector); the host reads the device once, at the end.  Under data parallelism
-    every rank evaluates its shard and gets the metric over all of them (see DetMetrics.compute)."""
+    every rank evaluates its shard and gets the metric over all of them (see DetMetrics.compute).
+    spike_stats=True: the windows are also counted by a spikes.SpikeStats, and the dict carries its "spikes/*" results
+    (firing rates, SynOps, dense MACs) over the whole evaluation."""
     from .infer import GraphedWindowDetector
     from .loss import pad_targets
     from .metrics import DetMetrics
@@ -206,13 +239,24 @@ def evaluate_model(model, dataloader, device, sequence_length=None, conf_thres=0
     model.to(device)
     metrics = DetMetrics(model.nc, device)
     detector = GraphedWindowDetector(model, conf_thres=conf_thres, iou_thres=iou_thres, multi_label=False, max_det=max_det)
-    for image_tensor, labels_tensor in dataloader:
-        if sequence_length is not None:
-            image_tensor = image_tensor[:, :sequence_length]
-        frames = image_tensor.to(device, non_blocking=True).contiguous()
-        rows, _, counts = detector(frames)
-        metrics.update(rows, counts, pad_targets(labels_tensor, frames.shape[0]), frames.shape[-2:])
-    return metrics.compute(_metrics_group(process_group))
+    prev_stats, stats = getattr(model, "spike_stats", None), None
+    if spike_stats:
+        from .spikes import MAX_T, SpikeStats
+        stats = SpikeStats(model, max_T=MAX_T)
+        model.spike_stats = stats
+    try:
+        for image_tensor, labels_tensor in dataloader:
+            if sequence_length is not None:
+                image_tensor = image_tensor[:, :sequence_length]
+            frames = image_tensor.to(device, non_blocking=True).contiguous()
+            rows, _, counts = detector(frames)
+            metrics.update(rows, counts, pad_targets(labels_tensor, frames.shape[0]), frames.shape[-2:])
+    finally:
+        model.spike_stats = prev_stats
+    res = metrics.compute(_metrics_group(process_group))
+    if stats is not None:
+        res.update((k, v) for k, v in stats.compute(_metrics_group(process_group)).items() if k.startswith("spikes/"))
+    return res
 
 
 # ------------------------------------------------------------------------------------------------

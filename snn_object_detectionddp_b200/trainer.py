@@ -121,7 +121,9 @@ class Trainer:
         The first `warmup_calls` calls run eagerly (they are real steps); the next call captures, then replays.
         Returned tensors are the graph's static outputs: read them before the next call."""
         padded = batch["padded"]
-        key = (tuple(frames.shape), frames.dtype, tuple(tuple(t.shape) for t in padded))
+        # attaching / detaching spike statistics changes the captured launches (counted LIF forwards): re-capture.  The key
+        # holds the stats object itself, so the counter buffer a captured graph adds into lives as long as the graph.
+        key = (tuple(frames.shape), frames.dtype, tuple(tuple(t.shape) for t in padded), getattr(self.model, "spike_stats", None))
         if self._graph_failed:
             return self.train_step(frames, {"padded": tuple(t.to(self.device) for t in padded)})
         if self._graph is not None and self._graph_key != key:
