@@ -222,6 +222,15 @@ int snn_adamw_step(float* p, float* g, float* m, float* v, void* shadow_bf16, lo
                    const float* hp, const double* sumsq, float* gnorm_out, int* step_ptr, int n_rows, int zero_grad,
                    void* stream);
 
+/* ---- exponential moving average of the weights (ultralytics ModelEMA.update, once per optimizer step):
+ *      e = d * e + (1 - d) * s over the flat fp32 master buffer ema[n] <- src[n] (n a multiple of 4, 16-byte aligned) and
+ *      over n_seg further fp32 segments, seg (device int64 [n_seg][3]) = {source address, destination address, length}
+ *      (BatchNorm running statistics, frozen parameters; any length).  decay (device fp32 [n_rows][2]) row k = {d, 1 - d} of update
+ *      k + 1; row min(*upd_ptr, n_rows - 1) is used and *upd_ptr is incremented afterwards (no host sync, CUDA-graph
+ *      replayable).  Products and sum rounded separately, as torch's `v *= d; v += (1 - d) * s`: bit-identical to it. ---- */
+int snn_ema_update(float* ema, const float* src, long long n, const long long* seg, int n_seg, const float* decay,
+                   int* upd_ptr, int n_rows, void* stream);
+
 /* ---- Detect decode (ultralytics Detect._inference, reached through model.py:209 in eval mode, and
  *      v8DetectionLoss.bbox_decode): boxes fp32 [N][4] in pixels (xywh != 0: cx,cy,w,h; else x1,y1,x2,y2) and
  *      sigmoid class probabilities fp32 [N][nc] (probs may be NULL). ---- */

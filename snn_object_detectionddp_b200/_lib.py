@@ -57,6 +57,7 @@ _SIGNATURES = {
     "snn_det_metrics_finalize": [_P, _P, _P, _L, _P, _I, _P, _P, _P, _P],
     "snn_grad_sumsq": [_P, _L, _P, _I, _P],
     "snn_adamw_step": [_P, _P, _P, _P, _P, _L, _P, _P, _P, _P, _I, _I, _P],
+    "snn_ema_update": [_P, _P, _L, _P, _I, _P, _P, _I, _P],
 }
 
 _lib = None

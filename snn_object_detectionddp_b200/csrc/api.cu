@@ -122,6 +122,7 @@ int launch_s2d8(const float*, __nv_bfloat16*, int, int, int, int, cudaStream_t);
 int launch_s2d8_u8(const uint8_t*, __nv_bfloat16*, int, int, int, int, cudaStream_t);
 int launch_adamw(float*, float*, float*, float*, __nv_bfloat16*, long long, const float*, const double*, float*,
                  int*, int, int, cudaStream_t);
+int launch_ema_update(float*, const float*, long long, const long long*, int, const float*, int*, int, cudaStream_t);
 int launch_bilinear(int, const __nv_bfloat16*, __nv_bfloat16*, int, int, int, int, int, int, cudaStream_t);
 int launch_pad_crop(const __nv_bfloat16*, __nv_bfloat16*, int, int, int, int, int, int, cudaStream_t);
 int launch_detect_decode(const float*, const float*, const float*, const float*, int, int, int, int, int, float*, float*, int,
@@ -307,6 +308,10 @@ int snn_grad_sumsq(const float* g, long long n, double* acc, int zero_first, voi
 int snn_adamw_step(float* p, float* g, float* m, float* v, void* shadow, long long n, const float* hp,
                    const double* sumsq, float* gnorm_out, int* step_ptr, int n_rows, int zero_grad, void* stream) {
     return launch_adamw(p, g, m, v, (__nv_bfloat16*)shadow, n, hp, sumsq, gnorm_out, step_ptr, n_rows, zero_grad, ST);
+}
+int snn_ema_update(float* ema, const float* src, long long n, const long long* seg, int n_seg, const float* decay,
+                   int* upd_ptr, int n_rows, void* stream) {
+    return launch_ema_update(ema, src, n, seg, n_seg, decay, upd_ptr, n_rows, ST);
 }
 int snn_detect_decode(const float* distri, const float* scores, const float* anchors, const float* stride, int B, int A,
                       int nc, int reg_max, int xywh, float* boxes, float* probs, void* stream) {

@@ -405,6 +405,69 @@ int launch_adamw(float* p, float* g, float* m, float* v, __nv_bfloat16* shadow, 
     return check_cuda(cudaGetLastError(), "adamw_kernel");
 }
 
+// ------------------------------------------------------------------------------------------
+// exponential moving average of the weights (ultralytics ModelEMA.update):  e = d * e + (1 - d) * s
+//   one float4 pass over the flat master buffer (12 B/param) + one block per BatchNorm running-statistics segment.
+// The decay comes from a host-computed table row {float(d), float(1 - d)} picked by a DEVICE update counter (as the
+// AdamW schedule row is), so a captured graph ramps the decay on replay.  __fmul_rn / __fadd_rn: the rounding and the
+// order of torch's `v *= d; v += (1 - d) * s` on fp32 tensors -- two products, one sum, never contracted into an FMA.
+// ------------------------------------------------------------------------------------------
+SNN_DEVINL float ema_mix(float e, float s, float d, float omd) { return __fadd_rn(__fmul_rn(e, d), __fmul_rn(omd, s)); }
+
+__global__ void __launch_bounds__(256)
+ema_flat_kernel(float* __restrict__ e, const float* __restrict__ s, long long n4, const float* __restrict__ decay,
+                const int* __restrict__ upd_ptr, int n_rows) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const float* row = decay + (size_t)min(*upd_ptr, n_rows - 1) * 2;
+    const float d = row[0], omd = row[1];
+    for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n4; i += (long long)gridDim.x * 256) {
+        const float4 ss = __ldg(reinterpret_cast<const float4*>(s) + i);
+        float4 ee = reinterpret_cast<float4*>(e)[i];
+        ee.x = ema_mix(ee.x, ss.x, d, omd);
+        ee.y = ema_mix(ee.y, ss.y, d, omd);
+        ee.z = ema_mix(ee.z, ss.z, d, omd);
+        ee.w = ema_mix(ee.w, ss.w, d, omd);
+        reinterpret_cast<float4*>(e)[i] = ee;
+    }
+}
+
+// seg = [n_seg][3] int64 {source address, destination address, length}; one block per segment, any length
+__global__ void __launch_bounds__(256)
+ema_segments_kernel(const long long* __restrict__ seg, const float* __restrict__ decay, const int* __restrict__ upd_ptr,
+                    int n_rows) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const float* row = decay + (size_t)min(*upd_ptr, n_rows - 1) * 2;
+    const float d = row[0], omd = row[1];
+    const float* __restrict__ s = reinterpret_cast<const float*>(seg[3 * blockIdx.x]);
+    float* __restrict__ e = reinterpret_cast<float*>(seg[3 * blockIdx.x + 1]);
+    const long long n = seg[3 * blockIdx.x + 2];
+    for (long long i = threadIdx.x; i < n; i += 256) e[i] = ema_mix(e[i], __ldg(s + i), d, omd);
+}
+
+int launch_ema_update(float* ema, const float* src, long long n, const long long* seg, int n_seg, const float* decay,
+                      int* upd_ptr, int n_rows, cudaStream_t st) {
+    SNN_REQUIRE(n % 4 == 0 && n >= 0, "ema_update: length %lld must be a multiple of 4", n);
+    SNN_REQUIRE(((uintptr_t)ema & 15) == 0 && ((uintptr_t)src & 15) == 0, "ema_update: buffers must be 16-byte aligned");
+    SNN_REQUIRE(decay && upd_ptr && n_rows >= 1, "ema_update: needs the decay table and the device update counter");
+    SNN_REQUIRE(n_seg >= 0 && (n_seg == 0 || seg), "ema_update: bad segment table");
+    const long long n4 = n / 4;
+    if (n4 > 0) {
+        long long blocks = (n4 + 255) / 256;
+        const long long cap = (long long)num_sms() * 8;
+        if (blocks > cap) blocks = cap;
+        launch_pdl(ema_flat_kernel, dim3((unsigned)blocks), dim3(256), 0, st, ema, src, n4, decay, upd_ptr, n_rows);
+        SNN_CUDA_OK(cudaGetLastError());
+    }
+    if (n_seg > 0) {
+        launch_pdl(ema_segments_kernel, dim3((unsigned)n_seg), dim3(256), 0, st, seg, decay, upd_ptr, n_rows);
+        SNN_CUDA_OK(cudaGetLastError());
+    }
+    launch_pdl(step_advance_kernel, dim3(1), dim3(1), 0, st, upd_ptr);
+    return check_cuda(cudaGetLastError(), "ema_update");
+}
+
 }  // namespace snn
 
 namespace snn {

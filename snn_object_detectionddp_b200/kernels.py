@@ -396,6 +396,30 @@ def adamw_step(p, g, m, v, shadow, hp, sumsq, gnorm_out=None, step=None, zero_gr
          work=("byte", (28.0 + (2.0 if shadow is not None else 0.0)) * p.numel()))
 
 
+def ema_update(ema, src, decay, updates, segments=None, segment_elems=0):
+    """ema = d * ema + (1 - d) * src (fp32, flat, length a multiple of 4), and the same over every (src, dst, n) row of
+    `segments` (device int64 [n_seg, 3] of addresses and lengths; `segment_elems` = the sum of the lengths, for the byte
+    count).  decay: device fp32 [rows, 2] = {d, 1 - d} per update; updates: device int32 counter picking the row (clamped
+    to the last), incremented by the call."""
+    require_cuda(ema, src, decay, updates, segments)
+    for name, t in (("ema", ema), ("src", src)):
+        if t.dtype != torch.float32 or not t.is_contiguous():
+            raise ValueError(f"ema_update: {name} must be a contiguous fp32 tensor")
+    if ema.numel() != src.numel():
+        raise ValueError(f"ema_update: {ema.numel()} averaged elements, {src.numel()} source elements")
+    if decay.dtype != torch.float32 or decay.dim() != 2 or decay.shape[1] != 2 or not decay.is_contiguous():
+        raise ValueError("ema_update: decay must be a contiguous fp32 [rows, 2] table")
+    if updates.dtype != torch.int32 or updates.numel() != 1:
+        raise ValueError("ema_update: updates must be a one-element int32 device counter")
+    n_seg = 0
+    if segments is not None:
+        if segments.dtype != torch.int64 or segments.dim() != 2 or segments.shape[1] != 3 or not segments.is_contiguous():
+            raise ValueError("ema_update: segments must be a contiguous int64 [n, 3] table")
+        n_seg = segments.shape[0]
+    call("snn_ema_update", ptr(ema), ptr(src), ema.numel(), ptr(segments), n_seg, ptr(decay), ptr(updates), decay.shape[0],
+         stream_ptr(), work=("byte", 12.0 * (ema.numel() + segment_elems)))
+
+
 # ---------------------------------------------------------------------------------------------
 # Detect-head depthwise conv, frame packer
 # ---------------------------------------------------------------------------------------------

@@ -94,8 +94,10 @@ class ParamStore:
                 and p.data_ptr() == self.flat_p.data_ptr() + 4 * e.offset
                 and p.stride() == e.logical_view(self.flat_p).stride())
 
-    def ensure(self, device):
-        """(Re)build the flat buffers on `device` and point every Parameter at its slice."""
+    def ensure(self, device, optimizer_state=True):
+        """(Re)build the flat buffers on `device` and point every Parameter at its slice.  optimizer_state=False: masters
+        and bf16 operand copies only -- no gradient or Adam-moment buffers (a model that is never trained, e.g. the
+        weight average of ema.ModelEMA)."""
         device = torch.device(device)
         if device.type != "cuda" and not getattr(K, "_EMULATED", False):
             raise K._lib.SnnKernelError("parameters must live on a CUDA device (no CPU fallback)")
@@ -110,11 +112,12 @@ class ParamStore:
         for e in self.entries:
             e.logical_view(flat_p).copy_(e.param.data.to(device=device, dtype=torch.float32))
         self.flat_p = flat_p
-        self.flat_g = torch.zeros(self.total, device=device, dtype=torch.float32)
         self.grads_clean = True
-        keep = old_m is not None and old_m.device == device
-        self.flat_m = old_m if keep else torch.zeros(self.total, device=device, dtype=torch.float32)
-        self.flat_v = old_v if keep else torch.zeros(self.total, device=device, dtype=torch.float32)
+        if optimizer_state:
+            self.flat_g = torch.zeros(self.total, device=device, dtype=torch.float32)
+            keep = old_m is not None and old_m.device == device
+            self.flat_m = old_m if keep else torch.zeros(self.total, device=device, dtype=torch.float32)
+            self.flat_v = old_v if keep else torch.zeros(self.total, device=device, dtype=torch.float32)
         self.shadow = torch.zeros(self.total, device=device, dtype=torch.bfloat16)
         self.device = device
         for e in self.entries:

@@ -108,9 +108,10 @@ def train_one_epoch(trainer, dataloader, sequence_length=None, writer=None, epoc
 
 @torch.no_grad()
 def validate_one_epoch(trainer, dataloader, sequence_length=None, writer=None, epoch=0, log_every=50, max_boxes=None,
-                       metrics=None):
+                       metrics=None, model=None):
     """reference train.py:106-146: eval mode, state reset per window, loss on the last frame.  `metrics`: a
-    metrics.DetMetrics that also receives the detections of the same forwards (call its compute() afterwards)."""
+    metrics.DetMetrics that also receives the detections of the same forwards (call its compute() afterwards).
+    `model`: the network to validate (default trainer.model; trainer.ema.ema validates the weight average)."""
     det_metrics = metrics
     metrics = DeviceMetrics(trainer.device, log_every)
     n_batches = len(dataloader)
@@ -119,7 +120,7 @@ def validate_one_epoch(trainer, dataloader, sequence_length=None, writer=None, e
             image_tensor = image_tensor[:, :sequence_length]
         frames = image_tensor.to(trainer.device, non_blocking=True)
         batch = _batch_dict(trainer, labels_tensor, frames.shape[0], max_boxes)
-        items = trainer.validate_step(frames.contiguous(), batch, metrics=det_metrics)
+        items = trainer.validate_step(frames.contiguous(), batch, metrics=det_metrics, model=model)
         if metrics.update(items, epoch * n_batches + batch_idx):
             _log_batches(writer, metrics.flush(), False)
     _log_batches(writer, metrics.flush(), False)
@@ -127,7 +128,7 @@ def validate_one_epoch(trainer, dataloader, sequence_length=None, writer=None, e
 
 
 def train_loop(model, train_loader, val_loader, config, device, save_dir, process_group=None, writer=None, log_every=50, graphed=False,
-               max_boxes=None, eval_map=False, spike_stats=False):
+               max_boxes=None, eval_map=False, spike_stats=False, ema=False):
     """reference train.py:148-241: epochs of train + validation, `latest.pt` every epoch and `best.pt` on improvement (the
     reference's checkpoint dict, plus optimizer state), the reference's epoch-level TensorBoard tags.
     eval_map=True: the validation forwards also feed a DetMetrics, and metrics/{precision,recall,mAP50,mAP50-95}(B) are
@@ -135,6 +136,10 @@ def train_loop(model, train_loader, val_loader, config, device, save_dir, proces
     spike_stats=True: one spikes.SpikeStats counts every forward of the loop; after each phase of an epoch it is read and
     reset, and Spikes/{train,val}_rate, Spikes/{train,val}_synops_fraction and the per-layer validation rates
     (Spikes_Val_Rate) are logged.  The model's previous `spike_stats` is restored on return.
+    ema=True: an ema.ModelEMA (ultralytics' defaults) is updated after every optimizer step, and each epoch's validation --
+    Loss/val and its components, metrics/*(B), the validation spike rates -- runs on the averaged weights, as ultralytics'
+    trainer does; best.pt is chosen by that loss and both checkpoints carry the average under 'ema'.  The trainer's
+    previous `ema` is restored on return.
     Returns the Trainer (the reference returns None)."""
     from .trainer import Trainer
     if writer is None:
@@ -158,6 +163,12 @@ def train_loop(model, train_loader, val_loader, config, device, save_dir, proces
         from .spikes import MAX_T, SpikeStats
         stats = SpikeStats(model, max_T=MAX_T)       # one buffer for both phases: the training graph is captured once
         model.spike_stats = stats
+    prev_ema, val_model = trainer.ema, model
+    if ema:
+        from .ema import ModelEMA
+        trainer.ema = ModelEMA(model)
+        val_model = trainer.ema.ema
+        val_model.spike_stats = stats
     log = writer is not None and rank0
     best_val_loss = float("inf")
     try:
@@ -175,7 +186,7 @@ def train_loop(model, train_loader, val_loader, config, device, save_dir, proces
             if det_metrics is not None:
                 det_metrics.reset()
             val_loss, val_comps = validate_one_epoch(trainer, val_loader, seq_len, writer=writer, epoch=epoch, log_every=log_every,
-                                                     max_boxes=max_boxes, metrics=det_metrics)
+                                                     max_boxes=max_boxes, metrics=det_metrics, model=val_model)
             if stats is not None:
                 res = _spike_results(stats, process_group)
                 if log:
@@ -202,6 +213,9 @@ def train_loop(model, train_loader, val_loader, config, device, save_dir, proces
                     trainer.save_checkpoint(os.path.join(str(save_dir), "best.pt"), epoch=epoch, best_val_loss=best_val_loss)
     finally:
         model.spike_stats = prev_stats
+        if val_model is not model:
+            val_model.spike_stats = None
+        trainer.ema = prev_ema
     return trainer
 
 

@@ -62,6 +62,8 @@ class Trainer:
         self._sumsq = torch.zeros(1, device=self.device, dtype=torch.float64)
         self.grad_norm = torch.zeros(1, device=self.device, dtype=torch.float32)
         self._ones3 = torch.ones(3, device=self.device, dtype=torch.float32)
+        # ema.ModelEMA: while set, every optimizer step also updates this weight average (captured graphs key on it)
+        self.ema = None
         self.group = process_group
         self.world = dist.get_world_size(process_group) if dist.is_initialized() else 1
         self.bucketer = None
@@ -111,6 +113,8 @@ class Trainer:
         K.adamw_step(st.flat_p, st.flat_g, st.flat_m, st.flat_v, st.shadow, self.hp, self._sumsq, self.grad_norm,
                      step=self._step_dev, zero_grad=True)
         st.grads_clean = True            # the optimizer pass zeroed the gradient buffer (next step's zero_grad is free)
+        if self.ema is not None:
+            self.ema.update()
         st.opt_epoch += 1
         self.step_idx += 1
 
@@ -121,9 +125,11 @@ class Trainer:
         The first `warmup_calls` calls run eagerly (they are real steps); the next call captures, then replays.
         Returned tensors are the graph's static outputs: read them before the next call."""
         padded = batch["padded"]
-        # attaching / detaching spike statistics changes the captured launches (counted LIF forwards): re-capture.  The key
-        # holds the stats object itself, so the counter buffer a captured graph adds into lives as long as the graph.
-        key = (tuple(frames.shape), frames.dtype, tuple(tuple(t.shape) for t in padded), getattr(self.model, "spike_stats", None))
+        # attaching / detaching spike statistics (counted LIF forwards) or a weight average (one more launch behind the
+        # optimizer) changes the captured launches: re-capture.  The key holds both objects, so the buffers a captured graph
+        # writes live as long as the graph.
+        key = (tuple(frames.shape), frames.dtype, tuple(tuple(t.shape) for t in padded), getattr(self.model, "spike_stats", None),
+               self.ema)
         if self._graph_failed:
             return self.train_step(frames, {"padded": tuple(t.to(self.device) for t in padded)})
         if self._graph is not None and self._graph_key != key:
@@ -148,6 +154,8 @@ class Trainer:
                 return self.train_step(frames, {"padded": tuple(t.to(self.device) for t in padded)})
             self.step_idx -= 1                 # capture records the launches without running them
             self.store.opt_epoch -= 1
+            if self.ema is not None:
+                self.ema.advanced(-1)
             self._graph, self._graph_key, self._static_out = g, key, out
         st = self.store
         if tuple(e.param._version for e in st.entries) != st._versions:
@@ -158,16 +166,19 @@ class Trainer:
         self._graph.replay()
         self.step_idx += 1
         st.opt_epoch += 1
+        if self.ema is not None:
+            self.ema.advanced(1)               # the replay ran the update kernel: the average's bf16 operands are stale
         return self._static_out
 
     # ------------------------------------------------------------------------------------------
     @torch.no_grad()
-    def validate_step(self, frames, batch, metrics=None, conf_thres=0.001, iou_thres=0.6, max_det=300):
+    def validate_step(self, frames, batch, metrics=None, conf_thres=0.001, iou_thres=0.6, max_det=300, model=None):
         """validate_one_epoch's inner step (reference train.py:106-131): eval mode (BatchNorm running statistics, state
         reset per window), loss on the last frame, no gradient.  Returns loss.detach() [3] as a DEVICE tensor.
         metrics: a metrics.DetMetrics -- the same forward is also decoded, put through NMS (eval_2.py:108 settings) and
-        matched against the batch's targets, without a host synchronisation."""
-        model = self.model
+        matched against the batch's targets, without a host synchronisation.
+        model: the network to validate (default: the trained one; `self.ema.ema` validates the weight average)."""
+        model = self.model if model is None else model
         was_training = model.training
         model.eval()
         try:
@@ -186,16 +197,22 @@ class Trainer:
     def save_checkpoint(self, path, epoch=0, best_val_loss=float("inf")):
         """The reference's checkpoint dict (train.py:204-209: 'epoch', 'model_state_dict', 'best_val_loss') -- loadable
         by the reference's own `model.load_state_dict(ckpt['model_state_dict'])` for the temporal_unet / detection_head
-        keys -- plus what the reference forgets (optimizer moments, schedule position) under 'trainer_state'."""
+        keys -- plus what the reference forgets (optimizer moments, schedule position) under 'trainer_state', and with a
+        weight average attached its ModelEMA.state_dict() under 'ema' (ultralytics keeps it under 'ema' / 'updates')."""
         st = self.store
-        torch.save({"epoch": epoch, "model_state_dict": {k: v.detach().cpu().contiguous() for k, v in self.model.state_dict().items()},
-                    "best_val_loss": best_val_loss,
-                    "trainer_state": {"step_idx": self.step_idx, "total_steps": self.total_steps,
-                                      "exp_avg": st.flat_m.cpu(), "exp_avg_sq": st.flat_v.cpu(),
-                                      "layout": [(e.name, e.offset, e.numel) for e in st.entries]}}, path)
+        ck = {"epoch": epoch, "model_state_dict": {k: v.detach().cpu().contiguous() for k, v in self.model.state_dict().items()},
+              "best_val_loss": best_val_loss,
+              "trainer_state": {"step_idx": self.step_idx, "total_steps": self.total_steps,
+                                "exp_avg": st.flat_m.cpu(), "exp_avg_sq": st.flat_v.cpu(),
+                                "layout": [(e.name, e.offset, e.numel) for e in st.entries]}}
+        if self.ema is not None:
+            ck["ema"] = self.ema.state_dict()
+        torch.save(ck, path)
 
     def load_checkpoint(self, path, strict=True):
-        """Accepts both this class's files and plain reference checkpoints (no 'trainer_state': moments restart at 0)."""
+        """Accepts both this class's files and plain reference checkpoints (no 'trainer_state': moments restart at 0).
+        The weight average is restored when the file and this trainer both have one; otherwise the file's 'ema' is ignored
+        and an attached average is left as it is (ultralytics' resume without 'ema')."""
         ck = torch.load(path, map_location="cpu", weights_only=False)
         self.model.load_state_dict(ck["model_state_dict"], strict=strict)
         st = self.store.ensure(self.device)
@@ -207,6 +224,8 @@ class Trainer:
             st.flat_v.copy_(ts["exp_avg_sq"])
             self.step_idx = int(ts["step_idx"])
             self._step_dev.fill_(self.step_idx)
+        if self.ema is not None and ck.get("ema") is not None:
+            self.ema.load_state_dict(ck["ema"])
         self._graph = None                       # captured graphs hold the old buffers' contents only by address: still valid, but re-capture is cheap and safe
         return ck.get("epoch", 0), ck.get("best_val_loss", float("inf"))
 
