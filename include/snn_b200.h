@@ -159,6 +159,20 @@ int snn_bn_act_bwd2(int pass, int act, const float* y, const float* scale, const
                     const float* invstd, const float* beta_bn, const float* v_init, const void* gs_bf16,
                     const float* gv_final, float* red, void* dy_bf16, float* gv_init, float* dgamma, float* dbeta,
                     int T, int P, int C, float beta, float theta, float alpha, void* stream);
+/* snn_bn_act_bwd2 with a per-layer addend of the spike gradient (spike-rate regularizer), LIF only (SiLU is an error):
+ * both passes use dL/ds = float(gs) + *ds_add in fp32 before the surrogate multiply, every element and timestep.  ds_add is a
+ * device pointer to ONE fp32 value (read on the device: CUDA-graph safe).  *ds_add == 0 gives snn_bn_act_bwd2's results. */
+int snn_bn_act_bwd2_ds(int pass, int act, const float* y, const float* scale, const float* shift, const float* mean,
+                       const float* invstd, const float* beta_bn, const float* v_init, const void* gs_bf16,
+                       const float* gv_final, float* red, void* dy_bf16, float* gv_init, float* dgamma, float* dbeta,
+                       int T, int P, int C, float beta, float theta, float alpha, const float* ds_add, void* stream);
+/* spike-rate regularizer of one step, one small launch: counts int64 [L][2][max_T] (spikes, neuron-steps; the SpikeStats
+ * layout), fanout fp64 [L] -> coef fp32 [L] (the snn_bn_act_bwd2_ds addend of each layer) and out fp32 [2 + L] =
+ * {P, phi, R_1..R_L}; P = a*max(0, phi - phi_max)^2 + (b/L)*sum_l max(0, r_min - R_l)^2, coef_l = B * dP/dS_l (DESIGN.md).
+ * fp64 in a fixed order, one rounding to fp32.  stats != NULL: counts of t < T are also added into stats [L][2][stats_max_T].
+ * L <= 64. */
+int snn_spike_reg_coef(const long long* counts, const double* fanout, int L, int max_T, double a, double phi_max, double r_min,
+                       double b, double B, float* coef, float* out, long long* stats, int stats_max_T, int T, void* stream);
 /* BN input gradient from gx and the reductions; dgamma/dbeta (+=) */
 int snn_bn_bwd_dx(const float* red, const float* gamma, const float* gx, const float* y,
                   const float* scale, const float* mean, const float* invstd, float* coef /*[T][2][C]*/,

@@ -15,7 +15,7 @@ ACT_LIF, ACT_SILU = 0, 1
 GEOM_TAPS = {GEOM_3x3_S1: 9, GEOM_3x3_S2: 9, GEOM_1x1: 1, GEOM_T2x2_S2: 4}
 
 _c = ctypes
-_P, _I, _L, _F = _c.c_void_p, _c.c_int, _c.c_longlong, _c.c_float
+_P, _I, _L, _F, _D = _c.c_void_p, _c.c_int, _c.c_longlong, _c.c_float, _c.c_double
 
 _SIGNATURES = {
     "snn_conv_fprop": [_I, _I, _I, _I, _P, _I, _L, _P, _I, _L, _P, _I, _I, _I, _I, _I, _P, _P, _I, _L, _I, _I, _P],
@@ -31,6 +31,8 @@ _SIGNATURES = {
     "snn_bn_act_fwd_count": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _L, _I, _I, _F, _F, _P],
     "snn_bn_act_bwd": [_I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _F, _F, _P],
     "snn_bn_act_bwd2": [_I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _F, _F, _P],
+    "snn_bn_act_bwd2_ds": [_I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _F, _F, _P, _P],
+    "snn_spike_reg_coef": [_P, _P, _I, _I, _D, _D, _D, _D, _D, _P, _P, _P, _I, _I, _P],
     "snn_bn_bwd_dx": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P],
     "snn_lstm_gates_fwd": [_P, _P, _P, _P, _P, _L, _I, _P],
     "snn_lstm_gates_bwd": [_P, _P, _P, _P, _P, _P, _P, _P, _L, _I, _P],

@@ -104,7 +104,9 @@ int launch_bn_act_bwd(int, int, const float*, const float*, const float*, const 
                       float, float, cudaStream_t);
 int launch_bn_act_bwd2(int, int, const float*, const float*, const float*, const float*, const float*, const float*,
                        const float*, const __nv_bfloat16*, const float*, float*, __nv_bfloat16*, float*, float*, float*, int, int,
-                       int, float, float, float, cudaStream_t);
+                       int, float, float, float, const float*, cudaStream_t);
+int launch_spike_reg_coef(const long long*, const double*, int, int, double, double, double, double, double, float*, float*,
+                          long long*, int, int, cudaStream_t);
 int launch_bn_bwd_dx(const float*, const float*, const float*, const float*, const float*, const float*, const float*, float*,
                      float*, float*, __nv_bfloat16*, int, int, int, cudaStream_t);
 int launch_lstm_gates_fwd(const float*, const float*, float*, float*, __nv_bfloat16*, long long, int, cudaStream_t);
@@ -251,7 +253,19 @@ int snn_bn_act_bwd2(int pass, int act, const float* y, const float* scale, const
                     float* red, void* dy, float* gv_init, float* dgamma, float* dbeta, int T, int P, int C, float beta,
                     float theta, float alpha, void* stream) {
     return launch_bn_act_bwd2(pass, act, y, scale, shift, mean, invstd, beta_bn, v_init, (const __nv_bfloat16*)gs, gv_final,
-                              red, (__nv_bfloat16*)dy, gv_init, dgamma, dbeta, T, P, C, beta, theta, alpha, ST);
+                              red, (__nv_bfloat16*)dy, gv_init, dgamma, dbeta, T, P, C, beta, theta, alpha, nullptr, ST);
+}
+int snn_bn_act_bwd2_ds(int pass, int act, const float* y, const float* scale, const float* shift, const float* mean,
+                       const float* invstd, const float* beta_bn, const float* v_init, const void* gs, const float* gv_final,
+                       float* red, void* dy, float* gv_init, float* dgamma, float* dbeta, int T, int P, int C, float beta,
+                       float theta, float alpha, const float* ds_add, void* stream) {
+    SNN_REQUIRE(ds_add != nullptr, "bn_act_bwd2_ds: ds_add (device pointer to the layer's dL/ds addend) is required");
+    return launch_bn_act_bwd2(pass, act, y, scale, shift, mean, invstd, beta_bn, v_init, (const __nv_bfloat16*)gs, gv_final,
+                              red, (__nv_bfloat16*)dy, gv_init, dgamma, dbeta, T, P, C, beta, theta, alpha, ds_add, ST);
+}
+int snn_spike_reg_coef(const long long* counts, const double* fanout, int L, int max_T, double a, double phi_max, double r_min,
+                       double b, double B, float* coef, float* out, long long* stats, int stats_max_T, int T, void* stream) {
+    return launch_spike_reg_coef(counts, fanout, L, max_T, a, phi_max, r_min, b, B, coef, out, stats, stats_max_T, T, ST);
 }
 int snn_bn_bwd_dx(const float* red, const float* gamma, const float* gx, const float* y, const float* scale,
                   const float* mean, const float* invstd, float* coef, float* dgamma, float* dbeta, void* dy, int T, int P,

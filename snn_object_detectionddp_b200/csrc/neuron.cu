@@ -551,7 +551,11 @@ SNN_DEVINL float ex2_approx(float x) {
 // EXACT: T == TMAX is a compile-time constant (no per-step guards; T = 1, 4, 8, 16 are the shapes on the path).
 // Coefficient tables are [channel pair][t] float4 rows with an odd row pitch of (TMAX|1) entries: a thread's T
 // entries sit at compile-time offsets from one base address and LDS.128 quarter-warps are bank-conflict free.
-template <int ACT, int TMAX, bool REDUCE, bool EXACT>
+// DS (LIF only, spike-rate regularizer): *ds_add (device fp32, one value for the whole layer) is added to every dL/ds in
+// fp32 before the surrogate multiply, in both passes.  Pass 1 reads it from the unused .z/.w of its tabB rows, pass 2 from
+// one shared-memory word behind the tables (a broadcast read), so neither keeps it in a register for the whole scan.  The
+// pointer is a trailing parameter: the instantiations without DS compile to the code they had without it.
+template <int ACT, int TMAX, bool REDUCE, bool EXACT, bool DS = false>
 __global__ void __launch_bounds__(256, (TMAX <= 4 ? 4 : (TMAX <= 8 ? 2 : 1)))
 bn_act_bwd2_kernel(const float* __restrict__ y, const float* __restrict__ scale, const float* __restrict__ shift,
                    const float* __restrict__ mean, const float* __restrict__ invstd, const float* __restrict__ beta_bn,
@@ -559,7 +563,8 @@ bn_act_bwd2_kernel(const float* __restrict__ y, const float* __restrict__ scale,
                    const float* __restrict__ gv_final, __nv_bfloat16* __restrict__ dy_out, float* __restrict__ gv_init,
                    float* __restrict__ red_out, float* dgamma, float* dbeta, int T_rt, int P, int C, int Cb, int pix_per_block,
                    float beta, float theta, float alpha, float invP,
-                   float* __restrict__ part /* REDUCE, deterministic mode: [gridDim.x][T*2*C] block partials, else null */) {
+                   float* __restrict__ part /* REDUCE, deterministic mode: [gridDim.x][T*2*C] block partials, else null */,
+                   const float* __restrict__ ds_add /* DS: the layer's dL/ds addend */) {
     pdl_launch_dependents();
     pdl_wait();
     extern __shared__ float4 shc4[];
@@ -571,14 +576,16 @@ bn_act_bwd2_kernel(const float* __restrict__ y, const float* __restrict__ scale,
     const int cg = threadIdx.x % tpp, row = threadIdx.x / tpp;
     float4* tabA = shc4;                                           // [tpp][PITCH] {scale.xy, shift.xy}
     float4* tabB = shc4 + tpp * PITCH;                             // REDUCE: {-mean.xy, 0, 0} ; DX: {-scale*mean(gx).xy, -mean(gx*xhat)*invstd.xy}
-    float* accum = reinterpret_cast<float*>(tabB + tpp * PITCH);   // REDUCE: [T][2][Cb]
+    float* accum = reinterpret_cast<float*>(tabB + tpp * PITCH);   // REDUCE: [T][2][Cb] ; DX with DS: the addend
+    const float cds = DS ? __ldg(ds_add) : 0.f;                    // REDUCE with DS: tabB = {-mean.xy, cds, cds}
+    if (DS && !REDUCE && threadIdx.x == 0) accum[0] = cds;
     for (int i = threadIdx.x; i < T * tpp; i += 256) {
         const int t = i / tpp, j = i % tpp, gc = t * C + c_base + 2 * j;
         const float2 sc = *reinterpret_cast<const float2*>(scale + gc), sh = *reinterpret_cast<const float2*>(shift + gc);
         tabA[j * PITCH + t] = make_float4(sc.x, sc.y, sh.x, sh.y);
         if (REDUCE) {
             const float2 m = *reinterpret_cast<const float2*>(mean + gc);
-            tabB[j * PITCH + t] = make_float4(-m.x, -m.y, 0.f, 0.f);
+            tabB[j * PITCH + t] = make_float4(-m.x, -m.y, cds, cds);
         } else {
             const float2 r0 = *reinterpret_cast<const float2*>(red_in + (t * 2 + 0) * C + c_base + 2 * j);
             const float2 r1 = *reinterpret_cast<const float2*>(red_in + (t * 2 + 1) * C + c_base + 2 * j);
@@ -665,7 +672,11 @@ bn_act_bwd2_kernel(const float* __restrict__ y, const float* __restrict__ scale,
 #pragma unroll
             for (int t = TMAX - 1; t >= 0; --t) {
                 if (EXACT || t < T) {
-                    const float2 g = f2(bf16_lo(gr[t]), bf16_hi(gr[t]));
+                    float2 g = f2(bf16_lo(gr[t]), bf16_hi(gr[t]));
+                    if (DS) {
+                        const float c = REDUCE ? tB[t].z : accum[0];
+                        g = __fadd2_rn(g, f2(c, c));
+                    }
                     const float2 uu = u[t];
                     float2 gx;
                     if (ACT == ACT_LIF) {
@@ -753,10 +764,11 @@ struct Bwd2Consts {
     float theta;
 };
 
-template <int ACT, bool REDUCE, int T0>
+template <int ACT, bool REDUCE, int T0, bool DS>
 SNN_DEVINL void bwd2_chunk8(const float2* __restrict__ yp, const uint32_t* __restrict__ gp, uint32_t* __restrict__ dp, size_t nt2,
                             const float4* tA, const float4* tB, float2 v, float2& gv, float2 nbb, const Bwd2Consts& k,
-                            float4* acc /* REDUCE: this thread's [16] accumulator slots in shared memory, stride 256 */) {
+                            float4* acc /* REDUCE: this thread's [16] accumulator slots in shared memory, stride 256 */,
+                            const float* cds /* DX with DS: the addend's shared-memory word */) {
     constexpr int TC = 8;
     float2 yv[TC];
     uint32_t gr[TC];
@@ -788,7 +800,11 @@ SNN_DEVINL void bwd2_chunk8(const float2* __restrict__ yp, const uint32_t* __res
     }
 #pragma unroll
     for (int t = TC - 1; t >= 0; --t) {
-        const float2 g = f2(bf16_lo(gr[t]), bf16_hi(gr[t]));
+        float2 g = f2(bf16_lo(gr[t]), bf16_hi(gr[t]));
+        if (DS) {
+            const float c = REDUCE ? tB[T0 + t].z : *cds;
+            g = __fadd2_rn(g, f2(c, c));
+        }
         const float2 uu = u[t];
         float2 gx;
         if (ACT == ACT_LIF) {
@@ -822,14 +838,15 @@ SNN_DEVINL void bwd2_chunk8(const float2* __restrict__ yp, const uint32_t* __res
     }
 }
 
-template <int ACT, bool REDUCE>
+template <int ACT, bool REDUCE, bool DS = false>
 __global__ void __launch_bounds__(256, 2)
 bn_act_bwd2_t16_kernel(const float* __restrict__ y, const float* __restrict__ scale, const float* __restrict__ shift,
                        const float* __restrict__ mean, const float* __restrict__ invstd, const float* __restrict__ beta_bn,
                        const float* __restrict__ red_in, const float* __restrict__ v_init, const __nv_bfloat16* __restrict__ gs,
                        const float* __restrict__ gv_final, __nv_bfloat16* __restrict__ dy_out, float* __restrict__ gv_init,
                        float* __restrict__ red_out, float* dgamma, float* dbeta, int T_rt, int P, int C, int Cb, int pix_per_block,
-                       float beta, float theta, float alpha, float invP, float* __restrict__ part /* as in bn_act_bwd2_kernel */) {
+                       float beta, float theta, float alpha, float invP, float* __restrict__ part /* as in bn_act_bwd2_kernel */,
+                       const float* __restrict__ ds_add /* as in bn_act_bwd2_kernel */) {
     pdl_launch_dependents();
     pdl_wait();
     extern __shared__ float4 shc4[];
@@ -841,13 +858,15 @@ bn_act_bwd2_t16_kernel(const float* __restrict__ y, const float* __restrict__ sc
     float4* tabA = shc4;
     float4* tabB = shc4 + tpp * PITCH;
     float* accum = reinterpret_cast<float*>(tabB + tpp * PITCH);
+    const float cds = DS ? __ldg(ds_add) : 0.f;
+    if (DS && !REDUCE && threadIdx.x == 0) accum[0] = cds;
     for (int i = threadIdx.x; i < T * tpp; i += 256) {
         const int t = i / tpp, j = i % tpp, gc = t * C + c_base + 2 * j;
         const float2 sc = *reinterpret_cast<const float2*>(scale + gc), sh = *reinterpret_cast<const float2*>(shift + gc);
         tabA[j * PITCH + t] = make_float4(sc.x, sc.y, sh.x, sh.y);
         if (REDUCE) {
             const float2 m = *reinterpret_cast<const float2*>(mean + gc);
-            tabB[j * PITCH + t] = make_float4(-m.x, -m.y, 0.f, 0.f);
+            tabB[j * PITCH + t] = make_float4(-m.x, -m.y, cds, cds);
         } else {
             const float2 r0 = *reinterpret_cast<const float2*>(red_in + (t * 2 + 0) * C + c_base + 2 * j);
             const float2 r1 = *reinterpret_cast<const float2*>(red_in + (t * 2 + 1) * C + c_base + 2 * j);
@@ -916,8 +935,8 @@ bn_act_bwd2_t16_kernel(const float* __restrict__ y, const float* __restrict__ sc
             }
             float2 gv = f2(0.f, 0.f);
             if (ACT == ACT_LIF && gv_final) gv = __ldg(reinterpret_cast<const float2*>(gv_final) + e2);
-            bwd2_chunk8<ACT, REDUCE, 8>(yp, gp, dp, nt2, tA, tB, v8, gv, nbb, k, acc);
-            bwd2_chunk8<ACT, REDUCE, 0>(yp, gp, dp, nt2, tA, tB, v0, gv, nbb, k, acc);
+            bwd2_chunk8<ACT, REDUCE, 8, DS>(yp, gp, dp, nt2, tA, tB, v8, gv, nbb, k, acc, accum);
+            bwd2_chunk8<ACT, REDUCE, 0, DS>(yp, gp, dp, nt2, tA, tB, v0, gv, nbb, k, acc, accum);
             if (!REDUCE && ACT == ACT_LIF && gv_init) *(reinterpret_cast<float2*>(gv_init) + e2) = gv;
         }
         if (REDUCE && !part) {
@@ -1178,6 +1197,82 @@ int launch_bn_act_fwd_count(const float* y, const float* scale, const float* shi
     return check_cuda(cudaGetLastError(), "bn_act_fwd_kernel<LIF, count>");
 }
 
+// ------------------------------------------------------------------------------------------
+// spike-rate regularizer (spikes.SpikeRateLoss): penalty, SynOps fraction, per-layer rates and the per-layer dL/ds addend
+// from one step's exact counts, one block.  counts [L][2][max_T] int64 (spikes, neuron-steps), fanout [L] fp64.
+//   S_l, N_l = sums over t;  R_l = S_l / N_l;  phi = sum_l F_l S_l / sum_l F_l N_l = sum_l F_l S_l / D
+//   P = a * max(0, phi - phi_max)^2 + (b / L) * sum_l max(0, r_min - R_l)^2
+//   c_l = B * (2a * max(0, phi - phi_max) * F_l / D - (2b / L) * max(0, r_min - R_l) / N_l)   (= B * dP/dS_l)
+// fp64 throughout in a fixed order with every product and sum rounded separately (no contraction), each result rounded
+// once to fp32: deterministic, and equal to the same expressions evaluated left to right in fp64 on the host.  A layer
+// with N_l = 0 has R_l = 0 and no rate term; D = 0 gives phi = 0.  stats != NULL: the step's counts of t < T are also
+// added into a SpikeStats buffer [L][2][stats_max_T] (one launch serves both).
+// ------------------------------------------------------------------------------------------
+constexpr int kRegMaxL = 64;
+__global__ void __launch_bounds__(kRegMaxL)
+spike_reg_coef_kernel(const long long* __restrict__ counts, const double* __restrict__ fanout, int L, int max_T, double a,
+                      double phi_max, double r_min, double b, double B, float* __restrict__ coef, float* __restrict__ out,
+                      long long* __restrict__ stats, int stats_max_T, int T) {
+    pdl_launch_dependents();
+    pdl_wait();
+    __shared__ double s_S[kRegMaxL], s_N[kRegMaxL], s_hp, s_D;
+    const int l = threadIdx.x;
+    if (l < L) {
+        long long s = 0, n = 0;
+        for (int t = 0; t < max_T; ++t) { s += counts[(l * 2 + 0) * max_T + t]; n += counts[(l * 2 + 1) * max_T + t]; }
+        s_S[l] = (double)s;
+        s_N[l] = (double)n;
+    }
+    if (stats) {
+        for (int i = threadIdx.x; i < L * 2 * T; i += blockDim.x) {
+            const int row = i / T, t = i % T;
+            stats[(size_t)row * stats_max_T + t] += counts[(size_t)row * max_T + t];
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double num = 0.0, den = 0.0, pr = 0.0;
+        for (int i = 0; i < L; ++i) {
+            num = __dadd_rn(num, __dmul_rn(fanout[i], s_S[i]));
+            den = __dadd_rn(den, __dmul_rn(fanout[i], s_N[i]));
+        }
+        for (int i = 0; i < L; ++i) {
+            if (s_N[i] > 0.0) {
+                const double h = fmax(0.0, __dadd_rn(r_min, -__ddiv_rn(s_S[i], s_N[i])));
+                pr = __dadd_rn(pr, __dmul_rn(h, h));
+            }
+        }
+        const double phi = den > 0.0 ? __ddiv_rn(num, den) : 0.0;
+        const double hp = fmax(0.0, __dadd_rn(phi, -phi_max));
+        out[0] = (float)__dadd_rn(__dmul_rn(__dmul_rn(a, hp), hp), __dmul_rn(__ddiv_rn(b, (double)L), pr));
+        out[1] = (float)phi;
+        s_hp = hp;
+        s_D = den;
+    }
+    __syncthreads();
+    if (l < L) {
+        const double n = s_N[l];
+        const double r = n > 0.0 ? __ddiv_rn(s_S[l], n) : 0.0;
+        const double h = n > 0.0 ? fmax(0.0, __dadd_rn(r_min, -r)) : 0.0;
+        const double u = s_D > 0.0 ? __ddiv_rn(__dmul_rn(__dmul_rn(__dmul_rn(2.0, a), s_hp), fanout[l]), s_D) : 0.0;
+        const double v = n > 0.0 ? __ddiv_rn(__dmul_rn(__ddiv_rn(__dmul_rn(2.0, b), (double)L), h), n) : 0.0;
+        coef[l] = (float)__dmul_rn(B, __dadd_rn(u, -v));
+        out[2 + l] = (float)r;
+    }
+}
+
+int launch_spike_reg_coef(const long long* counts, const double* fanout, int L, int max_T, double a, double phi_max, double r_min,
+                          double b, double B, float* coef, float* out, long long* stats, int stats_max_T, int T, cudaStream_t st) {
+    SNN_REQUIRE(L >= 1 && L <= kRegMaxL, "spike_reg_coef: L=%d layers must be in [1,%d]", L, kRegMaxL);
+    SNN_REQUIRE(max_T >= 1, "spike_reg_coef: max_T=%d must be >= 1", max_T);
+    SNN_REQUIRE(counts && fanout && coef && out, "spike_reg_coef: counts, fanout, coef and out are required");
+    SNN_REQUIRE(!stats || (T >= 0 && T <= max_T && T <= stats_max_T),
+                "spike_reg_coef: T=%d must fit both count buffers (max_T=%d, stats_max_T=%d)", T, max_T, stats_max_T);
+    launch_pdl(spike_reg_coef_kernel, dim3(1), dim3(kRegMaxL), 0, st, counts, fanout, L, max_T, a, phi_max, r_min, b, B, coef,
+               out, stats, stats_max_T, T);
+    return check_cuda(cudaGetLastError(), "spike_reg_coef_kernel");
+}
+
 template <int ACT, int TMAX, bool TRAIN>
 static int launch_bwd_t(const float* y, const float* scale, const float* shift, const float* mean, const float* invstd,
                         const float* v_init, const __nv_bfloat16* gs, const float* gv_final, float* gx,
@@ -1213,11 +1308,11 @@ int launch_bn_act_bwd(int act, int training, const float* y, const float* scale,
 }
 
 static int g_t16_chunked = 1; // 0: T == 16 uses the one-chunk kernel (A/B timing, snn_debug_set(9, 1))
-template <int ACT, int TMAX, bool REDUCE>
+template <int ACT, int TMAX, bool REDUCE, bool DS>
 static int launch_bwd2_t(const float* y, const float* scale, const float* shift, const float* mean, const float* invstd,
                          const float* beta_bn, const float* red_in, const float* v_init, const __nv_bfloat16* gs,
                          const float* gv_final, __nv_bfloat16* dy, float* gv_init, float* red_out, float* dgamma, float* dbeta,
-                         int T, int P, int C, float beta, float theta, float alpha, cudaStream_t st) {
+                         int T, int P, int C, float beta, float theta, float alpha, const float* ds_add, cudaStream_t st) {
     // bytes of shared memory per channel: two float4 tables per channel PAIR with pitch (TMAX|1), + REDUCE accumulators
     const int per_c = (TMAX | 1) * 16 + (REDUCE ? T * 8 : 0);
     const bool chunked = TMAX == 16 && T == 16 && g_t16_chunked;
@@ -1247,20 +1342,21 @@ static int launch_bwd2_t(const float* y, const float* scale, const float* shift,
         if (!part) return 2;
         if (!acc_slots) det_slots = sizeof(float) * (size_t)rows * T * 2 * Cb;
     }
-    const size_t smem = (size_t)Cb * per_c + acc_slots + det_slots;
+    const size_t ds_word = (DS && !REDUCE) ? 16 : 0;                                // DX pass: the addend behind the tables
+    const size_t smem = (size_t)Cb * per_c + acc_slots + det_slots + ds_word;
     SNN_REQUIRE(smem <= 200 * 1024, "bn_act_bwd2: %zu bytes of shared memory (C=%d T=%d)", smem, C, T);
 #define SNN_GO(EX)                                                                                                         \
     do {                                                                                                                   \
-        auto kern = bn_act_bwd2_kernel<ACT, TMAX, REDUCE, EX>;                                                             \
+        auto kern = bn_act_bwd2_kernel<ACT, TMAX, REDUCE, EX, DS>;                                                         \
         if (smem > 48 * 1024) SNN_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
         launch_pdl(kern, grid, dim3(256), smem, st, y, scale, shift, mean, invstd, beta_bn, red_in, v_init, gs, gv_final, dy, gv_init,   \
-                                      red_out, dgamma, dbeta, T, P, C, Cb, ppb, beta, theta, alpha, 1.0f / (float)P, part); \
+                                      red_out, dgamma, dbeta, T, P, C, Cb, ppb, beta, theta, alpha, 1.0f / (float)P, part, ds_add); \
     } while (0)
     if (chunked) {
-        auto kern = bn_act_bwd2_t16_kernel<ACT, REDUCE>;
+        auto kern = bn_act_bwd2_t16_kernel<ACT, REDUCE, DS>;
         if (smem > 48 * 1024) SNN_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         launch_pdl(kern, grid, dim3(256), smem, st, y, scale, shift, mean, invstd, beta_bn, red_in, v_init, gs, gv_final, dy, gv_init,
-                   red_out, dgamma, dbeta, T, P, C, Cb, ppb, beta, theta, alpha, 1.0f / (float)P, part);
+                   red_out, dgamma, dbeta, T, P, C, Cb, ppb, beta, theta, alpha, 1.0f / (float)P, part, ds_add);
     } else if (T == TMAX) SNN_GO(true); else SNN_GO(false);
 #undef SNN_GO
     SNN_CUDA_OK(cudaGetLastError());
@@ -1275,12 +1371,14 @@ void neuron_debug_set(int k, int v) {
 }
 
 // pass = 0: reduce (writes red [T][2][C], zeroed here); pass = 1: dx (reads red; writes dy, gv_init; dgamma/dbeta +=)
+// ds_add != NULL (LIF only): device fp32 addend of every dL/ds (spike-rate regularizer), the DS instantiations
 int launch_bn_act_bwd2(int pass, int act, const float* y, const float* scale, const float* shift, const float* mean,
                        const float* invstd, const float* beta_bn, const float* v_init, const __nv_bfloat16* gs,
                        const float* gv_final, float* red, __nv_bfloat16* dy, float* gv_init, float* dgamma, float* dbeta,
-                       int T, int P, int C, float beta, float theta, float alpha, cudaStream_t st) {
+                       int T, int P, int C, float beta, float theta, float alpha, const float* ds_add, cudaStream_t st) {
     SNN_REQUIRE(C % 2 == 0 && C >= 2, "bn_act_bwd2: C=%d must be even", C);
     SNN_REQUIRE(T >= 1 && T <= 16, "bn_act_bwd2: T=%d must be in [1,16]", T);
+    SNN_REQUIRE(ds_add == nullptr || act == ACT_LIF, "bn_act_bwd2_ds: the dL/ds addend needs the LIF neuron (act=%d)", act);
     if (pass == 0) SNN_CUDA_OK(cudaMemsetAsync(red, 0, sizeof(float) * 2 * T * C, st));
     if (act == ACT_SILU && T == 1 && g_t1_fast) {
         int Cb = C;
@@ -1310,15 +1408,18 @@ int launch_bn_act_bwd2(int pass, int act, const float* y, const float* scale, co
         if (part) return launch_ordered_combine_f32(part, (int)grid.x, 2LL * C, red, st);
         return 0;
     }
-#define SNN_BWD2(ACT, TM)                                                                                                   \
-    return pass == 0 ? launch_bwd2_t<ACT, TM, true>(y, scale, shift, mean, invstd, beta_bn, nullptr, v_init, gs, gv_final,   \
-                                                    nullptr, nullptr, red, nullptr, nullptr, T, P, C, beta, theta, alpha, st) \
-                     : launch_bwd2_t<ACT, TM, false>(y, scale, shift, mean, invstd, beta_bn, red, v_init, gs, gv_final, dy,   \
-                                                     gv_init, nullptr, dgamma, dbeta, T, P, C, beta, theta, alpha, st)
-    if (act == ACT_LIF) {
-        if (T == 1) SNN_BWD2(ACT_LIF, 1); else if (T <= 4) SNN_BWD2(ACT_LIF, 4); else if (T <= 8) SNN_BWD2(ACT_LIF, 8); else SNN_BWD2(ACT_LIF, 16);
+#define SNN_BWD2(ACT, TM, DS)                                                                                                \
+    return pass == 0 ? launch_bwd2_t<ACT, TM, true, DS>(y, scale, shift, mean, invstd, beta_bn, nullptr, v_init, gs, gv_final, \
+                                                        nullptr, nullptr, red, nullptr, nullptr, T, P, C, beta, theta, alpha,  \
+                                                        ds_add, st)                                                           \
+                     : launch_bwd2_t<ACT, TM, false, DS>(y, scale, shift, mean, invstd, beta_bn, red, v_init, gs, gv_final, dy, \
+                                                         gv_init, nullptr, dgamma, dbeta, T, P, C, beta, theta, alpha, ds_add, st)
+    if (act == ACT_LIF && ds_add) {
+        if (T == 1) SNN_BWD2(ACT_LIF, 1, true); else if (T <= 4) SNN_BWD2(ACT_LIF, 4, true); else if (T <= 8) SNN_BWD2(ACT_LIF, 8, true); else SNN_BWD2(ACT_LIF, 16, true);
+    } else if (act == ACT_LIF) {
+        if (T == 1) SNN_BWD2(ACT_LIF, 1, false); else if (T <= 4) SNN_BWD2(ACT_LIF, 4, false); else if (T <= 8) SNN_BWD2(ACT_LIF, 8, false); else SNN_BWD2(ACT_LIF, 16, false);
     } else {
-        if (T == 1) SNN_BWD2(ACT_SILU, 1); else if (T <= 4) SNN_BWD2(ACT_SILU, 4); else if (T <= 8) SNN_BWD2(ACT_SILU, 8); else SNN_BWD2(ACT_SILU, 16);
+        if (T == 1) SNN_BWD2(ACT_SILU, 1, false); else if (T <= 4) SNN_BWD2(ACT_SILU, 4, false); else if (T <= 8) SNN_BWD2(ACT_SILU, 8, false); else SNN_BWD2(ACT_SILU, 16, false);
     }
 #undef SNN_BWD2
 }

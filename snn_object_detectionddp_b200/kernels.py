@@ -258,10 +258,17 @@ def bn_act_bwd(act, training, y, scale, shift, mean, invstd, gs, T, v_init=None,
 
 
 def bn_act_bwd_train(act, y, scale, shift, mean, invstd, beta_bn, gs, T, dgamma, dbeta, v_init=None, gv_final=None,
-                     want_gv_init=False, beta=0.5, theta=1.0, alpha=2.0):
+                     want_gv_init=False, beta=0.5, theta=1.0, alpha=2.0, ds_add=None):
     """Train-mode (batch-statistics) backward of BN -> LIF|SiLU in two recompute passes (no fp32 gx round trip).
-    Returns (dy bf16, gv_init | None, red [T][2][C]); dgamma / dbeta (fp32 [C]) are accumulated into."""
-    require_cuda(y, scale, shift, mean, invstd, beta_bn, gs, dgamma, dbeta, v_init, gv_final)
+    Returns (dy bf16, gv_init | None, red [T][2][C]); dgamma / dbeta (fp32 [C]) are accumulated into.
+    ds_add (LIF only): one-element fp32 device tensor added to every dL/ds in fp32 before the surrogate multiply
+    (snn_bn_act_bwd2_ds; the spike-rate regularizer's c_l)."""
+    require_cuda(y, scale, shift, mean, invstd, beta_bn, gs, dgamma, dbeta, v_init, gv_final, ds_add)
+    if ds_add is not None:
+        if act != ACT_LIF:
+            raise _lib.SnnKernelError("bn_act_bwd_train: ds_add needs the LIF neuron")
+        if ds_add.dtype != torch.float32 or ds_add.numel() != 1:
+            raise ValueError(f"ds_add: a one-element fp32 device tensor required, got {ds_add.dtype} {tuple(ds_add.shape)}")
     c = y.shape[-1]
     p = y.numel() // (T * c)
     dev = y.device
@@ -273,9 +280,34 @@ def bn_act_bwd_train(act, y, scale, shift, mean, invstd, beta_bn, gs, T, dgamma,
     args = (ptr(y), ptr(scale), ptr(shift), ptr(mean), ptr(invstd), ptr(beta_bn), ptr(v_init), ptr(gs), ptr(gv_final), ptr(red),
             ptr(dy), ptr(gv_init), ptr(dgamma), ptr(dbeta), T, p, c, float(beta), float(theta), float(alpha), stream_ptr())
     tag = f"T{T} n{p * c} C{c}"
+    if ds_add is not None:      # same bytes: the addend is one broadcast float
+        call("snn_bn_act_bwd2_ds", 0, act, *args[:-1], ptr(ds_add), args[-1], work=("byte", 6.0 * y.numel(), "reduce " + tag))
+        call("snn_bn_act_bwd2_ds", 1, act, *args[:-1], ptr(ds_add), args[-1], work=("byte", 8.0 * y.numel(), "dx " + tag))
+        return dy, gv_init, red
     call("snn_bn_act_bwd2", 0, act, *args, work=("byte", 6.0 * y.numel(), "reduce " + tag))   # reads y fp32 + gs bf16
     call("snn_bn_act_bwd2", 1, act, *args, work=("byte", 8.0 * y.numel(), "dx " + tag))       # reads y + gs, writes dy bf16
     return dy, gv_init, red
+
+
+def spike_reg_coef(counts, fanout, coef, out, synops_weight, synops_max, rate_min, rate_min_weight, batch_size, stats=None, T=0):
+    """Spike-rate regularizer of one step (spikes.SpikeRateLoss), one launch: counts int64 [L][2][max_T] and fanout fp64
+    [L] -> coef fp32 [L] (each layer's dL/ds addend) and out fp32 [2 + L] = (P, phi, R_1..R_L).  stats: a SpikeStats
+    counts buffer int64 [L][2][stats_max_T] that also receives counts[:, :, :T]."""
+    require_cuda(counts, fanout, coef, out, stats)
+    if counts.dtype != torch.int64 or counts.dim() != 3 or counts.shape[1] != 2 or not counts.is_contiguous():
+        raise ValueError(f"spike_reg_coef: counts must be contiguous int64 [L][2][max_T], got {counts.dtype} {tuple(counts.shape)}")
+    L, max_T = counts.shape[0], counts.shape[2]
+    for name, t, dt, n in (("fanout", fanout, torch.float64, L), ("coef", coef, torch.float32, L), ("out", out, torch.float32, L + 2)):
+        if t is None or t.dtype != dt or t.numel() != n or not t.is_contiguous():
+            raise ValueError(f"spike_reg_coef: {name} must be a contiguous {dt} tensor of {n} elements")
+    smt = 0
+    if stats is not None:
+        if stats.dtype != torch.int64 or tuple(stats.shape[:2]) != (L, 2) or stats.dim() != 3 or not stats.is_contiguous():
+            raise ValueError(f"spike_reg_coef: stats must be contiguous int64 [{L}][2][max_T], got {stats.dtype} {tuple(stats.shape)}")
+        smt = stats.shape[2]
+    call("snn_spike_reg_coef", ptr(counts), ptr(fanout), L, max_T, float(synops_weight), float(synops_max), float(rate_min),
+         float(rate_min_weight), float(batch_size), ptr(coef), ptr(out), ptr(stats), smt, int(T), stream_ptr(),
+         work=("byte", 8.0 * counts.numel() + 8.0 * L + 4.0 * (2 * L + 2) + (16.0 * L * T if stats is not None else 0.0)))
 
 
 def bn_bwd_dx(red, gamma, gx, y, scale, mean, invstd, dgamma, dbeta, T):

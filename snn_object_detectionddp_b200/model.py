@@ -41,6 +41,9 @@ class RunCtx:
         # dead frames.  None = every timestep is live.
         self.live_T = live_T
         self.spike_stats = None     # spikes.SpikeStats the LIF ConvBlocks count into (None: uncounted launches)
+        # spikes.SpikeRateLoss of a training step: the LIF ConvBlocks count into ITS per-step buffer (it hands the counts on to
+        # spike_stats) and their backward adds its per-layer coefficient to the spike gradient
+        self.spike_reg = None
 
 
 def _to_nhwc_bf16(x):
@@ -96,7 +99,10 @@ class ConvBlock(nn.Module):
             cfg["dead_grad_unread"] = getattr(rc, "dead_grad_unread", False)
         if slot_x0 is not None:
             cfg["slot_x0"] = slot_x0          # (GradSlot, 'first' | 'last'): see ops.GradSlot
-        if rc.spike_stats is not None and self.neuron.kind == "lif":
+        if rc.spike_reg is not None and self.neuron.kind == "lif":
+            cfg["spike_counts"] = rc.spike_reg.layer_counts(self._snn_name, rc.T)
+            cfg["spike_grad"] = rc.spike_reg.layer_grad(self._snn_name)
+        elif rc.spike_stats is not None and self.neuron.kind == "lif":
             cfg["spike_counts"] = rc.spike_stats.layer_counts(self._snn_name, rc.T)
         if self.geom == GEOM_3x3_S2 and ((x0.shape[1] | x0.shape[2]) & 1):
             # odd H or W (e.g. the 15x20 P5 level of a 480x640 frame): zero-pad to even -- the extra row / column is exactly
@@ -490,17 +496,24 @@ class YOLOTemporalUNet(nn.Module):
         return stats
 
     # ---- fused sequence path -------------------------------------------------------------
-    def forward_sequence(self, frames, hidden_state=None, return_state=False, all_steps=False, record=None):
+    def forward_sequence(self, frames, hidden_state=None, return_state=False, all_steps=False, record=None, spike_reg=None):
         """frames [B,T,3,H,W] fp32 on the GPU.  Returns (HeadOut of the LAST step as in train.py:64-66, hidden);
         `hidden` is None unless return_state (final LSTM state + LIF membranes, for streaming inference).
-        `record`: optional dict that receives every ConvBlock's output (spikes) by module name (flip-rate reports)."""
+        `record`: optional dict that receives every ConvBlock's output (spikes) by module name (flip-rate reports).
+        `spike_reg`: a spikes.SpikeRateLoss (train mode only) whose per-step counters this forward fills and whose
+        coefficients the backward adds to the LIF spike gradients (Trainer.train_step passes Trainer.spike_reg)."""
         B, T = frames.shape[0], frames.shape[1]
         stats = self._spike_stats_for(frames, T)
+        if spike_reg is not None:
+            if not self.training:
+                raise ValueError("spike_reg applies to train-mode forwards (the penalty enters the train-mode LIF backward)")
+            spike_reg.begin_forward(self.temporal_unet, T, self.feature_extractor.feature_hw(*frames.shape[-2:]), frames.device)
         st = store_for(self, frames.device)
         st.refresh_operands()
         feats = self.feature_extractor.forward_seq(frames, B, T)
         rc = RunCtx(st, T, want_state=return_state, live_T=None if (all_steps or not self.skip_dead_backward) else 1)
         rc.spike_stats = stats
+        rc.spike_reg = spike_reg
         # the head's inputs are produced by the U-Net output convs, which slice the dead frames' gradient away themselves:
         # head-internal gradients of the dead frames are never read and need no zero fill
         rc.dead_grad_unread = rc.live_T is not None

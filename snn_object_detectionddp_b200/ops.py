@@ -131,7 +131,7 @@ class ConvBNActFn(Function):
             dbeta = st.grad_view(cfg["bn"].bias)
             dy, gv0, _ = K.bn_act_bwd_train(neuron.act, y, scale, shift, mean, invstd, cfg["bn"].bias, gs, T, dgamma, dbeta,
                                             v_init=v_init, gv_final=gvf, want_gv_init=want_gv0, beta=neuron.beta,
-                                            theta=neuron.v_th, alpha=neuron.alpha)
+                                            theta=neuron.v_th, alpha=neuron.alpha, ds_add=cfg.get("spike_grad"))
             st.grad_done(cfg["bn"].weight)
             st.grad_done(cfg["bn"].bias)
         else:

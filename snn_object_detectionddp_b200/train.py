@@ -15,6 +15,7 @@ TensorBoard tags (train.py:88-100, 137-143, 211-226), unchanged:
     Loss/train_batch, Train_Loss_Components_Batch/{box,cls,dfl}_loss_batch, LearningRate/batch,
     Loss/val_batch, Val_Loss_Components_Batch/{box,cls,dfl}_loss_batch,
     Loss/train, Loss/val, LearningRate, Train_Loss_Components/{box,cls,dfl}_loss, Val_Loss_Components/{box,cls,dfl}_loss
+With a spike-rate regularizer (train_loop(spike_reg=...)) also Loss/train_spike_reg_batch and Loss/train_spike_reg.
 """
 import math
 import os
@@ -34,15 +35,17 @@ class DeviceMetrics:
     steps to the host once and returns [(global_step, items[3], lr, scalar)]; `averages(n_batches)` is the epoch return
     value of the reference: (total_loss / n, total_components / n).  `scale`: the reference's TRAINING scalar is
     `loss_components.sum()` with loss_components = loss * batch_size (train.py:74-75), its VALIDATION scalar is
-    `loss_components_detached.sum()` (train.py:127) -- scale = B resp. 1."""
+    `loss_components_detached.sum()` (train.py:127) -- scale = B resp. 1.
+    extra=True: one more per-step device scalar (`update(..., extra=)`, the spike-rate penalty) rides in the same ring and
+    read; flush() rows then carry it as a fifth element and `extra_average(n_batches)` is its epoch mean."""
 
-    def __init__(self, device, every=50):
-        self.device, self.every = torch.device(device), max(1, int(every))
-        self.total = torch.zeros(4, device=self.device, dtype=torch.float64)       # components[3], scalar
-        self.ring = torch.zeros(self.every, 5, device=self.device, dtype=torch.float32)
+    def __init__(self, device, every=50, extra=False):
+        self.device, self.every, self.extra = torch.device(device), max(1, int(every)), bool(extra)
+        self.total = torch.zeros(4 + self.extra, device=self.device, dtype=torch.float64)       # components[3], scalar[, extra]
+        self.ring = torch.zeros(self.every, 5 + self.extra, device=self.device, dtype=torch.float32)
         self.steps, self.n = [], 0
 
-    def update(self, items, global_step, lr=0.0, scale=1.0):
+    def update(self, items, global_step, lr=0.0, scale=1.0, extra=None):
         slot = len(self.steps)
         it = items.detach()
         self.ring[slot, :3].copy_(it, non_blocking=True)
@@ -50,6 +53,9 @@ class DeviceMetrics:
         self.ring[slot, 4] = it.sum() * scale
         self.total[:3] += it.double()
         self.total[3] += self.ring[slot, 4].double()
+        if self.extra:
+            self.ring[slot, 5].copy_(extra.detach().reshape(()), non_blocking=True)
+            self.total[4] += self.ring[slot, 5].double()
         self.steps.append(int(global_step))
         self.n += 1
         return len(self.steps) >= self.every
@@ -58,25 +64,31 @@ class DeviceMetrics:
         if not self.steps:
             return []
         host = self.ring[:len(self.steps)].cpu()          # the ONE synchronisation per `every` steps
-        out = [(g, host[i, :3].clone(), float(host[i, 3]), float(host[i, 4])) for i, g in enumerate(self.steps)]
+        out = [(g, host[i, :3].clone(), float(host[i, 3]), float(host[i, 4])) + ((float(host[i, 5]),) if self.extra else ())
+               for i, g in enumerate(self.steps)]
         self.steps = []
         return out
 
     def averages(self, n_batches):
-        tot = (self.total / max(1, n_batches)).float().cpu()
+        tot = (self.total[:4] / max(1, n_batches)).float().cpu()
         return float(tot[3]), tot[:3]
+
+    def extra_average(self, n_batches):
+        return float(self.total[4] / max(1, n_batches))
 
 
 def _log_batches(writer, rows, train):
     if writer is None:
         return
     tag_loss, tag_comp = ("Loss/train_batch", "Train_Loss_Components_Batch") if train else ("Loss/val_batch", "Val_Loss_Components_Batch")
-    for gstep, items, lr, scalar in rows:
+    for gstep, items, lr, scalar, *extra in rows:
         writer.add_scalar(tag_loss, scalar, gstep)
         writer.add_scalars(tag_comp, {"box_loss_batch": float(items[0]), "cls_loss_batch": float(items[1]),
                                       "dfl_loss_batch": float(items[2])}, gstep)
         if train:
             writer.add_scalar("LearningRate/batch", lr, gstep)
+            if extra:
+                writer.add_scalar("Loss/train_spike_reg_batch", extra[0], gstep)
 
 
 def _batch_dict(trainer, labels_tensor, batch_size, max_boxes):
@@ -86,9 +98,11 @@ def _batch_dict(trainer, labels_tensor, batch_size, max_boxes):
 def train_one_epoch(trainer, dataloader, sequence_length=None, writer=None, epoch=0, log_every=50, max_boxes=None, graphed=False,
                     prefetcher=None):
     """reference train.py:46-104.  `trainer` = trainer.Trainer (it owns model, loss, optimizer and schedule).
-    Returns (avg_loss, avg_loss_components[3]) like the reference."""
+    Returns (avg_loss, avg_loss_components[3]) like the reference.  With trainer.spike_reg set, its per-step penalty is
+    logged with the batch scalars and its epoch mean is left in trainer.spike_reg.epoch_mean."""
     trainer.model.train()
-    metrics = DeviceMetrics(trainer.device, log_every)
+    reg = trainer.spike_reg
+    metrics = DeviceMetrics(trainer.device, log_every, extra=reg is not None)
     n_batches = len(dataloader)
     step_fn = trainer.train_step_graphed if graphed else trainer.train_step
     for batch_idx, (image_tensor, labels_tensor) in enumerate(dataloader):
@@ -100,9 +114,12 @@ def train_one_epoch(trainer, dataloader, sequence_length=None, writer=None, epoc
         _, items = step_fn(frames.contiguous(), batch)
         # the reference logs loss_components.sum() = B * sum(items) as 'Loss/train_batch' and the detached per-image
         # components (train.py:74-95); `items` are those detached components
-        if metrics.update(items, epoch * n_batches + batch_idx, lr, scale=float(frames.shape[0])):
+        if metrics.update(items, epoch * n_batches + batch_idx, lr, scale=float(frames.shape[0]),
+                          extra=None if reg is None else reg.last[0]):
             _log_batches(writer, metrics.flush(), True)
     _log_batches(writer, metrics.flush(), True)
+    if reg is not None:
+        reg.epoch_mean = metrics.extra_average(n_batches)
     return metrics.averages(n_batches)
 
 
@@ -128,7 +145,7 @@ def validate_one_epoch(trainer, dataloader, sequence_length=None, writer=None, e
 
 
 def train_loop(model, train_loader, val_loader, config, device, save_dir, process_group=None, writer=None, log_every=50, graphed=False,
-               max_boxes=None, eval_map=False, spike_stats=False, ema=False):
+               max_boxes=None, eval_map=False, spike_stats=False, ema=False, spike_reg=None):
     """reference train.py:148-241: epochs of train + validation, `latest.pt` every epoch and `best.pt` on improvement (the
     reference's checkpoint dict, plus optimizer state), the reference's epoch-level TensorBoard tags.
     eval_map=True: the validation forwards also feed a DetMetrics, and metrics/{precision,recall,mAP50,mAP50-95}(B) are
@@ -140,6 +157,10 @@ def train_loop(model, train_loader, val_loader, config, device, save_dir, proces
     Loss/val and its components, metrics/*(B), the validation spike rates -- runs on the averaged weights, as ultralytics'
     trainer does; best.pt is chosen by that loss and both checkpoints carry the average under 'ema'.  The trainer's
     previous `ema` is restored on return.
+    spike_reg: a dict of spikes.SpikeRateLoss keywords (synops_weight, synops_max, rate_min, rate_min_weight); None reads
+    config["training"]["spike_reg"] when present.  Every training step then also minimises B times the spike-rate penalty,
+    and Loss/train_spike_reg_batch (with the batch scalars) and Loss/train_spike_reg (epoch mean) are logged.  The
+    trainer's previous `spike_reg` is restored on return.
     Returns the Trainer (the reference returns None)."""
     from .trainer import Trainer
     if writer is None:
@@ -163,6 +184,12 @@ def train_loop(model, train_loader, val_loader, config, device, save_dir, proces
         from .spikes import MAX_T, SpikeStats
         stats = SpikeStats(model, max_T=MAX_T)       # one buffer for both phases: the training graph is captured once
         model.spike_stats = stats
+    if spike_reg is None:
+        spike_reg = tc.get("spike_reg")
+    prev_reg = trainer.spike_reg
+    if spike_reg is not None:
+        from .spikes import MAX_T, SpikeRateLoss
+        trainer.spike_reg = SpikeRateLoss(model, **dict({"max_T": MAX_T}, **spike_reg))
     prev_ema, val_model = trainer.ema, model
     if ema:
         from .ema import ModelEMA
@@ -205,6 +232,8 @@ def train_loop(model, train_loader, val_loader, config, device, save_dir, proces
                 writer.add_scalar("Loss/train", train_loss, epoch)
                 writer.add_scalar("Loss/val", val_loss, epoch)
                 writer.add_scalar("LearningRate", trainer.lr(), epoch)
+                if trainer.spike_reg is not None:
+                    writer.add_scalar("Loss/train_spike_reg", trainer.spike_reg.epoch_mean, epoch)
                 writer.add_scalars("Train_Loss_Components", {k: float(v) for k, v in zip(COMPONENTS, train_comps)}, epoch)
                 writer.add_scalars("Val_Loss_Components", {k: float(v) for k, v in zip(COMPONENTS, val_comps)}, epoch)
             if val_loss < best_val_loss:
@@ -216,6 +245,7 @@ def train_loop(model, train_loader, val_loader, config, device, save_dir, proces
         if val_model is not model:
             val_model.spike_stats = None
         trainer.ema = prev_ema
+        trainer.spike_reg = prev_reg
     return trainer
 
 

@@ -64,6 +64,8 @@ class Trainer:
         self._ones3 = torch.ones(3, device=self.device, dtype=torch.float32)
         # ema.ModelEMA: while set, every optimizer step also updates this weight average (captured graphs key on it)
         self.ema = None
+        # spikes.SpikeRateLoss: while set, every training step also minimises B * its penalty (captured graphs key on it)
+        self.spike_reg = None
         self.group = process_group
         self.world = dist.get_world_size(process_group) if dist.is_initialized() else 1
         self.bucketer = None
@@ -92,13 +94,20 @@ class Trainer:
 
     def train_step(self, frames, batch):
         """frames fp32 [B,T,3,H,W] on the device; batch = {'batch_idx','cls','bboxes'} (train.py:68-72) or
-        prepare_batch(...).  Returns (loss*B [3], loss.detach() [3]) as DEVICE tensors."""
-        model, st = self.model, self.store
+        prepare_batch(...).  Returns (loss*B [3], loss.detach() [3]) as DEVICE tensors.
+        With `spike_reg` set, the forward counts into its per-step buffer (zeroed first), its coefficient launch runs before
+        the loss, and the LIF backward adds the coefficients to the spike gradients; the return value is unchanged (the
+        penalty is in spike_reg.last)."""
+        model, st, reg = self.model, self.store, self.spike_reg
         model.train()
         st.zero_grad()
         if self.bucketer is not None:
             self.bucketer.begin_step()
-        det, _ = model.forward_sequence(frames)
+        if reg is not None:
+            reg.begin_step()
+        det, _ = model.forward_sequence(frames, spike_reg=reg)
+        if reg is not None:
+            reg.finish_forward(frames.shape[0], frames.shape[1], getattr(model, "spike_stats", None))
         loss, items = self.loss_fn(det, batch)
         # = loss.sum().backward() of train.py:75-76 without the reduction / expand kernels
         torch.autograd.backward((loss,), (self._ones3,))
@@ -125,11 +134,11 @@ class Trainer:
         The first `warmup_calls` calls run eagerly (they are real steps); the next call captures, then replays.
         Returned tensors are the graph's static outputs: read them before the next call."""
         padded = batch["padded"]
-        # attaching / detaching spike statistics (counted LIF forwards) or a weight average (one more launch behind the
-        # optimizer) changes the captured launches: re-capture.  The key holds both objects, so the buffers a captured graph
-        # writes live as long as the graph.
+        # attaching / detaching spike statistics (counted LIF forwards), a weight average (one more launch behind the
+        # optimizer) or a spike-rate regularizer changes the captured launches: re-capture.  The key holds the objects, so the
+        # buffers a captured graph writes live as long as the graph.
         key = (tuple(frames.shape), frames.dtype, tuple(tuple(t.shape) for t in padded), getattr(self.model, "spike_stats", None),
-               self.ema)
+               self.ema, self.spike_reg)
         if self._graph_failed:
             return self.train_step(frames, {"padded": tuple(t.to(self.device) for t in padded)})
         if self._graph is not None and self._graph_key != key:
